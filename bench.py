@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the cube-transition hot path (BASELINE.json metric: cube transitions/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A *step* is one pass of the fused scramble (K1) over one batch: BASELINE.json configs[2],
@@ -752,6 +752,26 @@ def replay_own_rows(torch, ops, dev, size, moves, states, solved, reward, rank, 
     return ok, int(idx.size)
 
 
+DUMP_ROWS = 1 << 16
+
+
+def dump_outputs(path, torch, states, solved, reward, counters):
+    """`--dump-outputs DIR`: what the last timed step handed its caller, as float32 / float64 .npy files, so two
+    builds can be compared output for output.  The per-cube outputs are a fixed sample of DUMP_ROWS rows (seeded,
+    sorted; every row when there are no more), 15 MB at 8 Mi instances; `rows` holds their indices and `counters`
+    the step's exact [solved, produced] totals over all rows (over all ranks when N > 1)."""
+    import numpy as np
+    n = states.shape[0]
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.RandomState(0).choice(n, DUMP_ROWS, replace=False))
+    idx = torch.from_numpy(rows).to(states.device)
+    out = {"rows": rows.astype(np.float64), "states": states[idx].float().cpu().numpy(),
+           "solved": solved[idx].float().cpu().numpy(), "reward": reward[idx].float().cpu().numpy(),
+           "counters": counters[:2].double().cpu().numpy()}
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_b200_arm(args):
     import torch
     import rubiks_cube_solver_b200 as R
@@ -852,6 +872,8 @@ def run_b200_arm(args):
     barrier()                                             # ... and keep sampling until they are done
     clocks.recording = False
     clocks.__exit__(None, None, None)
+    if args.dump_outputs and rank == 0:                   # before the isolated launches below rewrite the buffers
+        dump_outputs(args.dump_outputs, torch, states, solved, reward, totals)
     local_step_s = e0.elapsed_time(e1) * 1e-3 / args.steps
     step_s = cdist.max_over_ranks(local_step_s, dev)
     # where a multi-GPU region's time goes: every rank's own kernels (GPUs of one box differ by ~1 %) and what
@@ -981,7 +1003,13 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-other", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true", help="N > 1: do not pin each rank to its GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's slice) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_b200_arm(args)

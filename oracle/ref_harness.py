@@ -4,8 +4,8 @@ The reference tree is read-only, exists only in the build container (never on
 the GPU box) and does not import as shipped; ``load_reference()`` applies the
 four test-only shims of SURVEY.md section 8c (stub gym, stub matplotlib,
 ``np.int``, stand-in ``assets/py222.py`` -- all under ``oracle/ref_shims/``)
-and returns the reference's modules.  Used by ``oracle/gen_golden.py`` and by
-``tests/test_oracle_vs_reference.py`` (which skips when the tree is absent).
+and returns the reference's modules.  Used by ``oracle/gen_golden.py`` and
+``oracle/gen_pin222.py``, which record its outputs under ``tests/golden/``.
 """
 import importlib
 import os

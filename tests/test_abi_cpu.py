@@ -221,3 +221,7 @@ def test_bench_scaling_modes_and_reference_arm_line():
     assert line["impl"] == "reference" and line["config"] == cfg and line["n_gpus"] == 8 and line["steps"] == 2
     assert line["value"] > 0 and line["e2e"]["value"] == line["value"] and line["cpu_baseline"]["kind"] == "port"
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["unit"] == "transitions/s" and line["higher_is_better"] is True
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py")] + bad, capture_output=True, text=True,
+                             timeout=300, cwd=root)
+        assert out.returncode == 2 and "error:" in out.stderr and not out.stdout

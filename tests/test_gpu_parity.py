@@ -1440,3 +1440,36 @@ def test_fallback_paths_under_ab_switches(switch):
                           "-p", "no:cacheprovider", "-k", k], capture_output=True, text=True, timeout=600, env=env, cwd=root)
     assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-2000:]
     assert " passed" in out.stdout and " failed" not in out.stdout
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: the last timed step's outputs (a seeded row sample, float32 / float64) equal the
+    oracle on the benchmark's own seeded moves, and the same arguments with another --steps write the same files."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    n, dumps = 70007, []
+    for steps in (2, 3):
+        d = str(tmp_path / ("steps%d" % steps))
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", str(steps),
+                              "--warmup", "1", "--instances-per-gpu", str(n), "--e2e-steps", "2", "--skip-cpu",
+                              "--skip-other", "--dump-outputs", d], capture_output=True, text=True, timeout=600, cwd=root)
+        assert out.returncode == 0, out.stderr[-3000:]
+        line = json.loads(out.stdout.strip().splitlines()[-1])
+        assert line["steps"] == steps and line["gpu_launches"] == steps
+        dumps.append({f[:-4]: np.load(os.path.join(d, f)) for f in os.listdir(d)})
+    a, b = dumps
+    assert sorted(a) == ["counters", "reward", "rows", "solved", "states"]
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64) and np.array_equal(a[k], b[k]), k
+    gen = torch.Generator(device=dev()).manual_seed(1234)
+    moves = torch.randint(0, 12, (n, 30), dtype=torch.uint8, device=dev(), generator=gen).cpu().numpy()
+    want = O.scramble(3, moves)
+    solved = O.is_solved(3, want)
+    rows = a["rows"].astype(np.int64)
+    assert rows.size == 1 << 16 and (np.diff(rows) > 0).all() and rows[-1] < n
+    assert (a["states"] == want[rows]).all() and (a["solved"] == solved[rows]).all()
+    assert (a["reward"] == O.rewards(solved[rows])).all()
+    assert a["counters"].tolist() == [int(solved.sum()), n]

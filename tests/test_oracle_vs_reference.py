@@ -1,55 +1,58 @@
-"""Oracle vs the reference's own code, imported live from /root/reference under the
-test-only shims (oracle/ref_harness.py).  Skipped where the tree is absent (GPU box)."""
+"""Oracle vs the reference's own outputs: the tables, step-by-step walks and seeded resets that
+oracle/gen_golden.py recorded from the reference's code (gym-cube's cube_env.py, assets/py333.py,
+utils.py) into tests/golden/."""
 import numpy as np
 import pytest
 
 from oracle import cube_np as O
-from oracle import ref_harness
 from oracle import tables as T
+from oracle.scalar_env import ScalarCubeEnv
 
-pytestmark = pytest.mark.skipif(not ref_harness.reference_available(),
-                                reason="/root/reference not present")
-
-
-@pytest.fixture(scope="module")
-def R():
-    return ref_harness.load_reference()
+from conftest import golden
 
 
-def test_tables_live(R):
-    p = R.py333
-    assert (p.moveDefs == T.MOVE_DEFS_3).all()
-    assert (p.corner_pieceDefs == T.CORNER_DEFS_3).all() and (p.edge_pieceDefs == T.EDGE_DEFS_3).all()
-    assert (p.corner_pieceInds == T.CORNER_INDS_3).all() and (p.edge_pieceInds == T.EDGE_INDS_3).all()
-    assert (p.corner_hashOP == T.CORNER_HASH_W).all() and (p.edge_hashOP == T.EDGE_HASH_W).all()
-    assert [p.moveInds[n] for n in T.ACTIONS[3]] == list(range(12))
-    assert R.utils.get_env_config(2) == ([7, 21], 6) and R.utils.get_env_config(3) == ([20, 24], 12)
+def test_tables_live():
+    g = golden("reference_tables.npz")
+    assert (g["moveDefs"] == T.MOVE_DEFS_3).all()
+    assert (g["corner_pieceDefs"] == T.CORNER_DEFS_3).all() and (g["edge_pieceDefs"] == T.EDGE_DEFS_3).all()
+    assert (g["corner_pieceInds"] == T.CORNER_INDS_3).all() and (g["edge_pieceInds"] == T.EDGE_INDS_3).all()
+    # corner_hashOP / edge_hashOP: the solved cube's pieces hash to their own slots, orientation 0
+    s = g["initState_3"].astype(np.int64)
+    assert (g["corner_pieceInds"][s[g["corner_pieceDefs"]] @ T.CORNER_HASH_W] == [[i, 0] for i in range(8)]).all()
+    assert (g["edge_pieceInds"][s[g["edge_pieceDefs"]] @ T.EDGE_HASH_W] == [[i, 0] for i in range(12)]).all()
+    # moveInds order and get_env_config (utils.py): the env's action names and observation shape
+    for size in (2, 3):
+        assert list(g["actions_%d" % size]) == T.ACTIONS[size] and len(T.ACTIONS[size]) == T.N_ACTIONS[size]
+        assert golden("config1_%d.npz" % size)["onehot"].shape[1:] == T.STATE_DIM[size]
+    assert (T.STATE_DIM[2], T.N_ACTIONS[2], T.STATE_DIM[3], T.N_ACTIONS[3]) == ((7, 21), 6, (20, 24), 12)
 
 
 @pytest.mark.parametrize("size", (2, 3))
-def test_random_walks_live(R, size):
-    env = R.make_env(size)
-    rng = np.random.RandomState(99)
-    A = T.N_ACTIONS[size]
-    moves = rng.randint(A, size=(40, 25))
+def test_random_walks_live(size):
+    g = golden("walks_%d.npz" % size)
+    moves = g["moves"]
+    n, d = moves.shape
     _, trail, flags = O.scramble(size, moves, per_step=True)
-    enc = O.encode(size, trail.reshape(40 * 25, -1)).reshape((40, 25) + T.STATE_DIM[size])
-    for w in range(40):
-        env.init_state()
-        for k in range(25):
-            obs, r, d, _ = env.step(int(moves[w, k]))
-            assert (env.sim_cube == trail[w, k]).all()
-            assert (obs == enc[w, k]).all()
-            assert d == flags[w, k] and r == (1.0 if d else -1.0)
+    enc = O.encode(size, trail.reshape(n * d, -1)).reshape((n, d) + T.STATE_DIM[size])
+    for w in range(n):
+        for k in range(d):
+            assert (g["stickers"][w, k] == trail[w, k]).all()
+            assert (g["onehot"][w, k] == enc[w, k]).all()
+            assert g["done"][w, k] == flags[w, k] and g["reward"][w, k] == (1.0 if flags[w, k] else -1.0)
+    assert g["done"].any()
 
 
 @pytest.mark.parametrize("size", (2, 3))
-def test_reset_live(R, size):
-    env = R.make_env(size)
-    for seed, depth in ((0, 1), (3, 7), (50, 30), (1023, 10)):
-        obs = env.reset(seed=seed, scramble_count=depth)
-        final = O.scramble(size, O.reference_moves(size, seed, depth)[None, :])
-        assert (env.sim_cube == final[0]).all()
-        assert (obs == O.encode(size, final)[0]).all()
+def test_reset_live(size):
+    g = golden("config1_%d.npz" % size)
+    depth = g["moves"].shape[1]
+    for seed in (0, 3, 50, 1023):
+        moves = O.reference_moves(size, seed, depth)
+        assert (moves == g["moves"][seed]).all()
+        final = O.scramble(size, moves[None, :])
+        assert (g["stickers"][seed] == final[0]).all()
+        assert (g["onehot"][seed] == O.encode(size, final)[0]).all()
+    saved = np.random.get_state()                              # the failing reset skips its set_state
     with pytest.raises(UnboundLocalError):
-        env.reset(seed=0, scramble_count=0)                  # cube_env.py:69
+        ScalarCubeEnv(size).reset(seed=0, scramble_count=0)    # cube_env.py:69
+    np.random.set_state(saved)

@@ -1,5 +1,5 @@
 import os, sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from rubiks_cube_solver_b200 import _lib
 if os.environ.get("AB_LIB"): _lib.LIB_PATH = os.environ["AB_LIB"]
