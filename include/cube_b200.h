@@ -268,6 +268,45 @@ int cube_decode(int cube_size, const void* onehot, int dtype, int encoding, int6
 int cube_validate_actions(int cube_size, const uint8_t* actions, int64_t count, uint64_t* counters,
                           void* stream);
 
+/* ---- exact 2x2x2 distances ----------------------------------------------------------------------
+ * The reference measures a solver by its solve percentage alone (test.py:103-158, train.py:167-198); the
+ * DeepCube line of work compares solution lengths with optimal ones.  The 2x2x2 of the reference (U, U', F,
+ * F', R, R', the DBL corner fixed) has 7! * 3^6 = 3 674 160 states, none more than 14 quarter turns from
+ * solved, so a table of every state's distance fits in 3.7 MB (resident in L2).
+ *
+ * Table layout: one uint8 distance per rank.  With (p_i, o_i) = py222 getOP of slot i = 0..6 (the pairs the
+ * 2x2x2 one-hot encoding is built from):
+ *     rank = L * 729 + T,   L = sum_{i=0..6} #{j > i : p_j < p_i} * (6 - i)!,   T = sum_{i=0..5} o_i * 3^(5 - i)
+ * o_6 is implied: the orientations of a reachable state sum to 0 mod 3.  The solved cube is rank 0.  A sticker
+ * row is REACHABLE exactly when the row rebuilt from its rank is the row; any other content (colours >= 6,
+ * hashes outside py222's table, two stickers swapped, a twisted corner) has distance CUBE_DISTANCE_UNREACHABLE.
+ * cube_size 3 returns CUBE_ERR_SIZE (its 4.3e19 states are out of reach).  A NULL table or states pointer, or
+ * n < 0, returns CUBE_ERR_ARG.  The table and sticker rows start on 16-byte boundaries; the byte outputs may start
+ * anywhere. */
+#define CUBE_DISTANCE_UNREACHABLE 255
+#define CUBE_DISTANCE_MAX_2 14
+
+/* number of table entries: 3 674 160 for cube_size 2 */
+int64_t cube_distance_table_entries(int cube_size);
+
+/* Fill table [cube_distance_table_entries] uint8 (caller-owned) with the distance of every rank: a
+ * level-synchronous breadth-first search from the solved cube, one launch per level. */
+int cube_distance_table_build(int cube_size, uint8_t* table, void* stream);
+
+/* distance [n] uint8 out: table[rank(states[i])], or CUBE_DISTANCE_UNREACHABLE.  states [n, 24] uint8. */
+int cube_distance(int cube_size, const uint8_t* table, const uint8_t* states, int64_t n, uint8_t* distance,
+                  void* stream);
+
+/* An optimal solution of every row, walking down the table: at every step the LOWEST action index whose child
+ * is one level closer.
+ *   actions_out [n, CUBE_DISTANCE_MAX_2] uint8  out  the solution, padded with CUBE_NOOP (cube_walk of the
+ *                                                     row with it ends solved for every reachable row)
+ *   length      [n]                     uint8  out  the solution's length = the distance (0 for a solved
+ *                                                     row); CUBE_DISTANCE_UNREACHABLE and only NOOPs for an
+ *                                                     unreachable row */
+int cube_solve_optimal(int cube_size, const uint8_t* table, const uint8_t* states, int64_t n, uint8_t* actions_out,
+                       uint8_t* length, void* stream);
+
 /* ---- host-buffer front end (end-to-end path) ------------------------------------------
  * For callers that hold NumPy / host arrays, as every caller of the reference does
  * (train.py:155, :186; test.py:123).  A pipeline handle owns a few stages of device

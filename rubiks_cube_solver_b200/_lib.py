@@ -15,12 +15,14 @@ SYMBOLS = (
     "cube_peer_buffer_bytes", "cube_peer_allreduce_i64",
     "cube_pipeline_create", "cube_pipeline_destroy", "cube_pipeline_scramble_host", "cube_pipeline_reset_host", "cube_host_alloc", "cube_host_free",
     "cube_env_host_create", "cube_env_host_destroy", "cube_env_host_step", "cube_env_host_scramble", "cube_env_host_encode",
+    "cube_distance_table_entries", "cube_distance_table_build", "cube_distance", "cube_solve_optimal",
 )
 
 ABI_VERSION = 2
 CUBE_ERR_SIZE, CUBE_ERR_ARG, CUBE_ERR_ALIGN, CUBE_ERR_ACTION = -1, -2, -3, -4
 DTYPE_BF16, DTYPE_F32, DTYPE_U8 = 0, 1, 2
 ENCODING_REFERENCE, ENCODING_EXACT = 0, 1
+DISTANCE_UNREACHABLE, DISTANCE_MAX_2 = 255, 14
 
 _lib = None
 
@@ -86,9 +88,14 @@ def load():
     lib.cube_env_host_step.argtypes = [vp, vp, ci, vp, vp, ctypes.POINTER(ci), vp]
     lib.cube_env_host_scramble.argtypes = [vp, vp, ci, vp, vp, ctypes.POINTER(ci), vp]
     lib.cube_env_host_encode.argtypes = [vp, vp, vp, vp]
+    lib.cube_distance_table_entries.argtypes = [ci]
+    lib.cube_distance_table_build.argtypes = [ci, vp, vp]
+    lib.cube_distance.argtypes = [ci, vp, vp, i64, vp, vp]
+    lib.cube_solve_optimal.argtypes = [ci, vp, vp, i64, vp, vp, vp]
     for name in SYMBOLS:
         if name not in ("cube_last_error",):
             getattr(lib, name).restype = ci
+    lib.cube_distance_table_entries.restype = i64
     if lib.cube_abi_version() != ABI_VERSION:
         raise CubeLibraryError("libcube_b200.so has ABI version %d, expected %d" % (lib.cube_abi_version(), ABI_VERSION))
     _lib = lib

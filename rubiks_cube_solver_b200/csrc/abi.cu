@@ -7,6 +7,7 @@
 
 #include "../../include/cube_b200.h"
 #include "cube_common.cuh"
+#include "cube_distance.cuh"
 #include "cube_kernels.h"
 
 namespace {
@@ -30,6 +31,13 @@ inline bool misaligned(const void* p) { return (reinterpret_cast<uintptr_t>(p) &
 inline bool misaligned4(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3u) != 0; }   // float / int32 arrays
 
 #define CUBE_CHECK_SIZE(fn) if (cube_size != 2 && cube_size != 3) return fail(CUBE_ERR_SIZE, fn)
+
+// the exact distance table exists for the 2x2x2 only
+int fail_distance_size(const char* what)
+{
+    snprintf(t_err, sizeof(t_err), "%s: exact distances exist for cube_size 2 only", what);
+    return CUBE_ERR_SIZE;
+}
 #define CUBE_DONE(fn, rc) do { int rc_ = (rc); return rc_ ? fail(rc_, fn) : 0; } while (0)
 
 }  // namespace
@@ -286,6 +294,39 @@ int cube_validate_actions(int cube_size, const uint8_t* actions, int64_t count, 
     if (misaligned(actions)) return fail(CUBE_ERR_ALIGN, "cube_validate_actions");
     CUBE_DONE("cube_validate_actions", cube::launch_validate(cube_size, actions, count,
                                                              (unsigned long long*)counters, (cudaStream_t)stream));
+}
+
+int64_t cube_distance_table_entries(int cube_size)
+{
+    if (cube_size != 2) return fail_distance_size("cube_distance_table_entries");
+    return (int64_t)kDist2Entries;
+}
+
+int cube_distance_table_build(int cube_size, uint8_t* table, void* stream)
+{
+    if (cube_size != 2) return fail_distance_size("cube_distance_table_build");
+    if (!table) return fail(CUBE_ERR_ARG, "cube_distance_table_build");
+    if (misaligned(table)) return fail(CUBE_ERR_ALIGN, "cube_distance_table_build");
+    CUBE_DONE("cube_distance_table_build", cube::launch_distance_build2(table, (cudaStream_t)stream));
+}
+
+int cube_distance(int cube_size, const uint8_t* table, const uint8_t* states, int64_t n, uint8_t* distance,
+                  void* stream)
+{
+    if (cube_size != 2) return fail_distance_size("cube_distance");
+    if (!table || !states || n < 0 || (n > 0 && !distance)) return fail(CUBE_ERR_ARG, "cube_distance");
+    if (misaligned(table) || misaligned(states)) return fail(CUBE_ERR_ALIGN, "cube_distance");
+    CUBE_DONE("cube_distance", cube::launch_distance2(table, states, n, distance, (cudaStream_t)stream));
+}
+
+int cube_solve_optimal(int cube_size, const uint8_t* table, const uint8_t* states, int64_t n, uint8_t* actions_out,
+                       uint8_t* length, void* stream)
+{
+    if (cube_size != 2) return fail_distance_size("cube_solve_optimal");
+    if (!table || !states || n < 0 || (n > 0 && (!actions_out || !length))) return fail(CUBE_ERR_ARG, "cube_solve_optimal");
+    if (misaligned(table) || misaligned(states)) return fail(CUBE_ERR_ALIGN, "cube_solve_optimal");
+    CUBE_DONE("cube_solve_optimal", cube::launch_solve_optimal2(table, states, n, actions_out, length,
+                                                                (cudaStream_t)stream));
 }
 
 }  // extern "C"

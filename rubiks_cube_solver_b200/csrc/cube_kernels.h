@@ -73,6 +73,13 @@ int launch_decode2(const void* onehot, int dtype, long long n, uint8_t* out, cud
 // 3x3x3 one-hot rows in the EXACT encoding -> sticker rows
 int launch_decode3_exact(const void* onehot, int dtype, long long n, uint8_t* out, cudaStream_t stream);
 
+// exact 2x2x2 distances (distance.cu, layout in cube_distance.cuh): the BFS table build (memsets and one launch
+// per level), the lookup and the optimal solve
+int launch_distance_build2(uint8_t* table, cudaStream_t stream);
+int launch_distance2(const uint8_t* table, const uint8_t* states, long long n, uint8_t* distance, cudaStream_t stream);
+int launch_solve_optimal2(const uint8_t* table, const uint8_t* states, long long n, uint8_t* actions, uint8_t* length,
+                          cudaStream_t stream);
+
 // one-shot SUM all-reduce of int64 values over peer-mapped exchange buffers (peer.cu)
 size_t peer_buffer_bytes(int cap);
 int launch_peer_allreduce_i64(int world, int rank, const uint64_t* peer_bufs, long long* values, int n, int cap,

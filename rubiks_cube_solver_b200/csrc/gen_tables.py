@@ -141,6 +141,17 @@ C_SRC_2, C_ROT_2 = cubie_action(MOVES_2, CORNER_SLOTS_2)
 assert all(E_ROT_3[m].sum() == 0 for m in (2, 3, 4, 5, 8, 9, 10, 11)), "only U/D may flip edges"
 assert all(E_ROT_3[m][4:8].sum() == 0 for m in range(12)), "middle-layer edges never flip"
 
+# 2x2x2 distance table (csrc/cube_distance.cuh): the cubies in py222 getOP's own terms -- slot q = the stickers
+# PIECE_DEFS_2[q], byte = cubelet | ori << 4 (kPieceCode2's format), a cubelet at ori o showing np.roll(home, o).
+# A turn moves the byte of slot src into slot q and adds (3 - rot) mod 3 to its ori.
+_D_SRC_2, _D_ROT_2 = cubie_action(MOVES_2, PIECE_DEFS_2)
+DIST_MOVE_2 = [int(_D_SRC_2[a][q]) | ((3 - int(_D_ROT_2[a][q])) % 3) << 4 for a in range(6) for q in range(7)]
+CUBIE_COLOURS_2 = [0] * 21      # 3 * cubelet + ori -> the colours the slot's stickers k = 0..2 show, one per byte
+for _p in range(7):
+    _c = [s // 4 for s in PIECE_DEFS_2[_p]]
+    for _o in range(3):
+        CUBIE_COLOURS_2[3 * _p + _o] = sum(_c[(k - _o) % 3] << (8 * k) for k in range(3))
+
 N_MOVE_ROWS = 16          # rows 0..A-1 = moves, the rest = identity (row 12 doubles as "no-op")
 W3 = 10                   # words per 3x3x3 move
 W2 = 4                    # words per 2x2x2 move
@@ -609,6 +620,10 @@ def render():
     o.append("// 2x2x2 decode (py222 getStickers): sticker positions of each slot, home colours of each cubelet\n")
     o.append(_c_array("uint8_t", "kPieceDefs2", [v for r in PIECE_DEFS_2 for v in r] + [14, 18, 23], per_line=24, fmt="%d"))
     o.append(_c_array("uint8_t", "kHomeColour2", [v // 4 for r in PIECE_DEFS_2 for v in r] + [3, 4, 5], per_line=24, fmt="%d"))
+    o.append("// 2x2x2 distance table (cube_distance.cuh): [move][slot] = source slot | ori added << 4, and\n"
+             "// [3 * cubelet + ori] = the colours of the slot's stickers k = 0..2, one per byte\n")
+    o.append(_c_array("uint8_t", "kDistMove2", DIST_MOVE_2, per_line=21, fmt="%d"))
+    o.append(_c_array("uint32_t", "kCubieColours2", CUBIE_COLOURS_2, per_line=7))
     return "".join(o)
 
 
@@ -726,6 +741,20 @@ def selftest(n=300, depth=37):
                 if m < n_act:
                     s = s[moves[m]]
             assert list(s) == emu(seq), "pair tables mishandle the no-move index"
+    # distance-table cubies: a turn through kDistMove2 equals getOP (hash -> kPieceCode2) of the turned stickers,
+    # and kCubieColours2 rebuilds the stickers
+    for _ in range(n):
+        s = np.repeat(np.arange(6), 4)
+        codes = list(range(7))
+        for m in rng.randint(6, size=depth):
+            s = s[MOVES_2[m]]
+            codes = [(codes[DIST_MOVE_2[7 * m + q] & 15] & 15)
+                     | (((codes[DIST_MOVE_2[7 * m + q] & 15] >> 4) + (DIST_MOVE_2[7 * m + q] >> 4)) % 3) << 4
+                     for q in range(7)]
+        assert codes == [PIECE_CODE_2[s[d[0]] + 2 * s[d[1]] + 10 * s[d[2]]] for d in PIECE_DEFS_2], \
+            "2x2x2 distance cubies disagree with getOP"
+        assert all(CUBIE_COLOURS_2[3 * (c & 15) + (c >> 4)] == sum(int(s[d[k]]) << (8 * k) for k in range(3))
+                   for c, d in zip(codes, PIECE_DEFS_2)), "kCubieColours2 does not rebuild the stickers"
     # cycles reproduce the gather rows
     for moves, cycles, n_s in ((MOVES_3, CYCLES_3, 54), (MOVES_2, CYCLES_2, 24)):
         for m in range(len(moves)):

@@ -387,6 +387,81 @@ def decode(cube_size, onehot, encoding="reference"):
     return out
 
 
+_distance_tables = {}
+_distance_lock = threading.Lock()
+
+
+def distance_table(device=None):
+    """The exact 2x2x2 distance table (C ABI cube_distance_table_build): uint8 [3674160], the quarter-turn
+    distance of every rank (layout in include/cube_b200.h).  Built on the device the first time it is asked for
+    there, then cached per device; treat it as read-only."""
+    dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    if dev.type != "cuda":
+        raise TypeError("distance_table lives on a CUDA device (this library has no CPU path)")
+    if dev.index is None:
+        dev = torch.device("cuda", torch.cuda.current_device())
+    with _distance_lock:
+        table = _distance_tables.get(dev.index)
+        if table is None:
+            lib = _lib.load()
+            table = torch.empty(_distance_entries(2), dtype=torch.uint8, device=dev)
+            with torch.cuda.device(dev):
+                _lib.check(lib.cube_distance_table_build(2, _ptr(table), _stream(dev)), "cube_distance_table_build")
+                torch.cuda.current_stream(dev).synchronize()              # once: callers on any stream may read it
+            _distance_tables[dev.index] = table
+    return table
+
+
+def _distance_entries(cube_size):
+    _geom(cube_size)
+    entries = _lib.load().cube_distance_table_entries(cube_size)
+    if entries < 0:
+        _lib.check(entries, "cube_distance_table_entries")                # 3x3x3: NotImplementedError
+    return entries
+
+
+def _distance_rows(cube_size, states):
+    _distance_entries(cube_size)
+    states = _require_cuda(states, "states")
+    n = states.shape[0]
+    if states.shape != (n, N_STICKERS[cube_size]):
+        raise ValueError("states must be [N, %d]" % N_STICKERS[cube_size])
+    return states, n, distance_table(states.device)
+
+
+def distance(cube_size, states, out=None):
+    """Exact distance of every sticker row (C ABI cube_distance): uint8 [N], 255 for a row that is not a
+    reachable state.  2x2x2 only (3x3x3 raises NotImplementedError)."""
+    states, n, table = _distance_rows(cube_size, states)
+    dev = states.device
+    if out is None:
+        out = torch.empty(n, dtype=torch.uint8, device=dev)
+    _require_cuda(out, "out")
+    if out.numel() != n:
+        raise ValueError("out must hold N = %d distances" % n)
+    if n:
+        with torch.cuda.device(dev):
+            _lib.check(_lib.load().cube_distance(cube_size, _ptr(table), _ptr(states), n, _ptr(out), _stream(dev)),
+                       "cube_distance")
+    return out
+
+
+def solve_optimal(cube_size, states):
+    """An optimal solution of every row (C ABI cube_solve_optimal): returns (actions uint8 [N, 14] padded with the
+    no-op index 12, length uint8 [N]); at every step the lowest action index whose child is one level closer.
+    `walk(cube_size, states, actions)` ends solved for every reachable row; an unreachable row gets length 255
+    and only no-ops.  2x2x2 only."""
+    states, n, table = _distance_rows(cube_size, states)
+    dev = states.device
+    actions = torch.empty((n, _lib.DISTANCE_MAX_2), dtype=torch.uint8, device=dev)
+    length = torch.empty(n, dtype=torch.uint8, device=dev)
+    if n:
+        with torch.cuda.device(dev):
+            _lib.check(_lib.load().cube_solve_optimal(cube_size, _ptr(table), _ptr(states), n, _ptr(actions),
+                                                      _ptr(length), _stream(dev)), "cube_solve_optimal")
+    return actions, length
+
+
 class HostCube(object):
     """One cube per call through host (NumPy) buffers -- C ABI cube_env_host_*: the per-call path of the
     drop-in CubeEnv (reset / step / get_obs, cube_env.py:56-147).  Two launches and one stream

@@ -116,3 +116,31 @@ def validation(model, cube_size, sample_scramble_count=30, sample_cube_count=10,
                        model_device=model_device)
     solved = res["solved"].view(len(depths), len(seeds)).float().mean(dim=1) * 100.0
     return [float(x) for x in solved.cpu()]
+
+
+def optimal_gap(model, seeds, depths, max_timesteps=200, mask_inverse=False, model_device=None):
+    """How far the greedy policy's 2x2x2 solutions are from optimal: `validation`'s solve-% curve with the
+    solution-length comparison beside it.  Every (depth, seed) cube is scrambled as reset(seed, depth) draws it and
+    solved by `greedy_solve`; the exact distance of every scramble comes from the distance table (ops.distance).
+
+    Returns one dict per depth: depth, solved_pct, mean_distance (over all cubes), mean_steps (over the cubes
+    greedy solved) and mean_excess (steps - distance over the cubes greedy solved, leaving out scrambles that
+    already end solved: greedy counts those only after stepping back, see the module docstring).  A mean over no
+    cube is NaN."""
+    seeds, depths = [int(s) for s in seeds], [int(d) for d in depths]
+    moves = reference_scrambles_device(2, seeds, depths)
+    res = greedy_solve(model, 2, moves, max_timesteps=max_timesteps, mask_inverse=mask_inverse,
+                       model_device=model_device)
+    start, _, _ = ops.scramble(2, moves, want_flags=False)
+    shape = (len(depths), len(seeds))
+    dist = ops.distance(2, start).cpu().numpy().reshape(shape).astype(np.int64)
+    solved = res["solved"].cpu().numpy().reshape(shape)
+    steps = res["steps"].cpu().numpy().reshape(shape)
+
+    def mean(x):
+        return float(x.mean()) if x.size else float("nan")
+
+    return [dict(depth=d, solved_pct=float(solved[i].mean()) * 100.0, mean_distance=mean(dist[i]),
+                 mean_steps=mean(steps[i][solved[i]]),
+                 mean_excess=mean((steps[i] - dist[i])[solved[i] & (dist[i] > 0)]))
+            for i, d in enumerate(depths)]
