@@ -32,8 +32,8 @@
  *     must be reproduced.
  *   - counters, when non-NULL, is uint64[4] on the device and is only ever
  *     ADDED to: [0] += outputs that are solved, [1] += outputs produced,
- *     [2] += out-of-range actions (cube_validate_actions), [3] += seeded rows that ran
- *     out of raw draws (cube_moves_from_seeds).
+ *     [2] += out-of-range actions (cube_validate_actions), [3] += seeded rows that needed
+ *     more than 227 raw draws (cube_moves_from_seeds; such rows are exact, see there).
  *     Rewards are +1.0f / -1.0f, so a reward total is 2*[0] - [1] exactly.
  */
 #ifndef CUBE_B200_H
@@ -110,8 +110,10 @@ int cube_peer_allreduce_i64(int world, int rank, const uint64_t* peer_buffers, i
  * legacy randint).  A shorter reset(seed, k') is the first k' entries of the row.
  *   seeds      [n]        uint32   in   (the reference's integer seeds, < 2^32)
  *   moves_out  [n, depth] uint8    out  depth <= 128
- * counters[3] += rows that would need more than 227 raw draws (practically never: > 7 sigma at depth
- * 128); such rows are padded with CUBE_NOOP. */
+ * A row is drawn from the first 227 raw outputs of its generator without materialising its state; a row
+ * those leave short (about one seed in 3e9 at depth 128: 2103926524 and 3830291768 for the 3x3x3,
+ * 3969546545 for the 2x2x2) continues from the full 624-word state, exactly as NumPy does, and
+ * counters[3] += 1 for it. */
 int cube_moves_from_seeds(int cube_size, const uint32_t* seeds, int64_t n, int depth, uint8_t* moves_out,
                           uint64_t* counters, void* stream);
 

@@ -2,51 +2,29 @@
 //   reset(seed, k):  np.random.seed(seed); np.random.randint(A, size=k)          cube_env.py:62-65
 // i.e. np.random.RandomState(seed).randint(A, size=k), for n seeds at once, so that seeded batches
 // (config 1: seeds 0..1023; validation: seed = 10 * cube, train.py:180) need no host RNG and no
-// upload of move bytes.
-//
-// NumPy's legacy generator is MT19937 seeded by init_genrand (mt[0] = seed, mt[j] = 1812433253 *
-// (mt[j-1] ^ mt[j-1] >> 30) + j) and randint(A) draws 32-bit outputs, masks them with the smallest
-// 2^b - 1 >= A - 1 and rejects values > A - 1 (numpy/random/_bounded_integers: masked rejection).
-// Output i < 227 of a freshly seeded generator only needs mt[i], mt[i+1] and mt[i+397] of the SEED
-// state, and those follow from a one-word recurrence -- so a thread keeps two running words (one at i,
-// one 397 ahead) and never materialises the 624-word state.  227 raw draws cover depth <= 128 with
-// > 7 sigma to spare (acceptance 3/4); a row that would need more is counted in counters[3] and padded
-// with CUBE_NOOP (the host wrapper raises).
+// upload of move bytes.  The per-seed draw -- a one-word-recurrence fast path for the first 227 raw
+// outputs and an exact slow path for the rare row that needs more -- is csrc/cube_seeds.cuh; a row that
+// took the slow path is counted in counters[3].
 #include <cuda_runtime.h>
 #include "cube_kernels.h"
 #include "../../include/cube_b200.h"
+#include "cube_seeds.cuh"
 
 namespace {
 
-// x >> K on the FMA pipe (IMAD.HI) instead of the ALU pipe (SHF): the recurrence and the tempering are
-// shift / xor / multiply chains.  Measured: 8 Mi seeds x depth 30 take 1.3 ms either way (3 390 warp
-// instructions per 32 seeds, ALU pipe 63 %, issue 59 %, `math_pipe_throttle` and `dispatch_stall` on top:
-// profiles/r01_k0_seeded_moves_ncu_summary.json) -- the 397 sequential seed-state steps and ~50 draw
-// iterations of ~35 instructions are what the generator costs (1.22 ms after the row stores stopped
-// rebuilding their address per draw); the fused scramble behind it takes 0.18 ms.
-template <int K>
-__device__ __forceinline__ uint32_t shr(uint32_t x)
-{
-    return __umulhi(x, 1u << (32 - K));
-}
-
-__device__ __forceinline__ uint32_t mt_next_seed_word(uint32_t prev, uint32_t j)
-{
-    return 1812433253u * (prev ^ shr<30>(prev)) + j;
-}
-
 constexpr int kSeedThreads = 128;
 
-// j as a constant-bank operand of the multiply-add (IMAD r, g, M, c[j]): with the loop index in a register
-// an unrolled step needs an extra ALU add for "+ j"
-struct SeedIndex { uint32_t v[400]; };
-constexpr SeedIndex make_seed_index()
-{
-    SeedIndex t{};
-    for (int j = 0; j < 400; ++j) t.v[j] = (uint32_t)j;
-    return t;
-}
-__constant__ SeedIndex kSeedIndex = make_seed_index();
+// a row of the CTA's shared-memory staging area as a 32-bit shared-window address that only ever advances: the
+// generic pointer form made the compiler rebuild the window base (S2R) for every accepted draw
+struct SharedRow {
+    uint32_t p, end;
+    __device__ __forceinline__ bool full() const { return p >= end; }
+    __device__ __forceinline__ void put(uint32_t v)
+    {
+        asm volatile("st.shared.u8 [%0], %1;" ::"r"(p), "r"(v) : "memory");
+        ++p;
+    }
+};
 
 __global__ void __launch_bounds__(kSeedThreads)
 seeded_moves_kernel(const uint32_t* __restrict__ seeds, long long n, int depth, uint32_t max_value, uint32_t mask,
@@ -59,36 +37,9 @@ seeded_moves_kernel(const uint32_t* __restrict__ seeds, long long n, int depth, 
     const long long base = (long long)blockIdx.x * kSeedThreads;
     const long long i = base + tid;
     if (i < n) {
-        const uint32_t seed = seeds[i];
-        uint32_t z = seed;
-#pragma unroll
-        for (int j = 1; j <= 397; ++j) z = mt_next_seed_word(z, kSeedIndex.v[j]);   // mt[397]: 3 instructions per step
-        uint32_t x = seed, xn = mt_next_seed_word(seed, 1), idx = 0;            // mt[0], mt[1]
-        // the row as a 32-bit shared-window address that only ever advances: the generic pointer form made
-        // the compiler rebuild the window base (S2R) for every accepted draw
-        uint32_t p = (uint32_t)__cvta_generic_to_shared(s_rows) + (uint32_t)(tid * depth);
-        const uint32_t end = p + (uint32_t)depth;
-        while (p < end && idx < 227) {
-            const uint32_t y = (x & 0x80000000u) | (xn & 0x7fffffffu);
-            uint32_t v = z ^ shr<1>(y) ^ ((y & 1u) ? 0x9908b0dfu : 0u);
-            v ^= shr<11>(v);
-            v ^= (v << 7) & 0x9d2c5680u;
-            v ^= (v << 15) & 0xefc60000u;
-            v ^= shr<18>(v);
-            ++idx;
-            x = xn;
-            xn = mt_next_seed_word(xn, idx + 1);
-            z = mt_next_seed_word(z, idx + 397);                                  // only used while idx + 397 <= 623
-            const uint32_t val = v & mask;
-            if (val <= max_value) {
-                asm volatile("st.shared.u8 [%0], %1;" ::"r"(p), "r"(val) : "memory");
-                ++p;
-            }
-        }
-        if (p < end) {
-            for (; p < end; ++p) asm volatile("st.shared.u8 [%0], %1;" ::"r"(p), "r"((uint32_t)CUBE_NOOP) : "memory");
-            if (counters) atomicAdd(&counters[3], 1ull);
-        }
+        const uint32_t p = (uint32_t)__cvta_generic_to_shared(s_rows) + (uint32_t)(tid * depth);
+        if (seed_row(seeds[i], max_value, mask, SharedRow{p, p + (uint32_t)depth}) && counters)
+            atomicAdd(&counters[3], 1ull);
     }
     __syncthreads();
     const long long rows = (n - base) < (long long)kSeedThreads ? (n - base) : (long long)kSeedThreads;
@@ -109,8 +60,7 @@ int launch_seeded_moves(int size, const uint32_t* seeds, long long n, int depth,
 {
     if (n == 0 || depth == 0) return 0;
     const uint32_t max_value = size == 3 ? 11u : 5u;
-    uint32_t mask = max_value;                                                   // smallest 2^b - 1 >= max_value
-    mask |= mask >> 1; mask |= mask >> 2; mask |= mask >> 4; mask |= mask >> 8; mask |= mask >> 16;
+    const uint32_t mask = seed_mask(max_value);
     const long long blocks = (n + kSeedThreads - 1) / kSeedThreads;
     seeded_moves_kernel<<<(unsigned)blocks, kSeedThreads, (size_t)kSeedThreads * depth, stream>>>(seeds, n, depth, max_value,
                                                                                                    mask, moves, counters);

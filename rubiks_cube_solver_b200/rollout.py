@@ -38,8 +38,9 @@ def reference_scrambles_device(cube_size, seeds, depths, device=None):
     and padded with the no-op index.  uint8 [len(depths) * len(seeds), max(depths)] on the device."""
     depths = list(depths)
     dmax = max(depths)
-    if dmax > 128:
-        return torch.from_numpy(reference_scrambles(cube_size, seeds, depths)).to(device)
+    if dmax > 128:                                                                     # deeper than K0 draws
+        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        return torch.from_numpy(reference_scrambles(cube_size, seeds, depths)).to(dev)
     base = ops.moves_from_seeds(cube_size, seeds, dmax, device=device)                  # [S, dmax]
     d = torch.tensor(depths, device=base.device).view(-1, 1, 1)
     k = torch.arange(dmax, device=base.device).view(1, 1, -1)
