@@ -1,7 +1,5 @@
 // extern "C" boundary of libcube_b200.so: argument checks, then the launchers.
 // See include/cube_b200.h for the contract of every entry point.
-#include <atomic>
-#include <cstdlib>
 #include <cstdio>
 #include <cuda_runtime.h>
 
@@ -9,6 +7,7 @@
 #include "cube_common.cuh"
 #include "cube_distance.cuh"
 #include "cube_kernels.h"
+#include "cube_launch.cuh"
 
 namespace {
 
@@ -42,49 +41,6 @@ int fail_distance_size(const char* what)
 
 }  // namespace
 
-namespace cube {
-
-static int g_reserved_sms = -1;          // -1: take CUBE_RESERVED_SMS (default 0)
-
-int reserved_sms()
-{
-    if (g_reserved_sms < 0) {
-        const char* e = getenv("CUBE_RESERVED_SMS");
-        g_reserved_sms = e ? atoi(e) : 0;
-        if (g_reserved_sms < 0) g_reserved_sms = 0;
-    }
-    return g_reserved_sms;
-}
-
-int device_slot()
-{
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0) dev = 0;
-    return dev & 63;
-}
-
-int persistent_ctas()
-{
-    const int n = sm_count() - reserved_sms();
-    return n < 1 ? 1 : n;
-}
-
-int sm_count()
-{
-    static std::atomic<int> cached[64];   // per device, 0 = not asked yet (host threads may drive different devices)
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 148;
-    std::atomic<int>& c = cached[dev & 63];
-    int v = c.load(std::memory_order_relaxed);
-    if (v == 0) {
-        if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || v < 1) v = 148;
-        c.store(v, std::memory_order_relaxed);
-    }
-    return v;
-}
-
-}  // namespace cube
-
 extern "C" {
 
 int cube_abi_version(void) { return CUBE_ABI_VERSION; }
@@ -96,7 +52,7 @@ int cube_sm_count(void) { return cube::sm_count(); }
 int cube_set_reserved_sms(int n)
 {
     if (n < 0) return fail(CUBE_ERR_ARG, "cube_set_reserved_sms");
-    cube::g_reserved_sms = n;
+    cube::set_reserved_sms(n);
     return CUBE_OK;
 }
 

@@ -10,6 +10,7 @@
 // One thread per parent; the A child values are read as 16-byte vectors (A*4 = 48 / 24 bytes).
 #include <cuda_runtime.h>
 #include "cube_kernels.h"
+#include "cube_launch.cuh"
 
 namespace {
 

@@ -7,7 +7,8 @@
 #include "../../include/cube_b200.h"
 
 // counters layout (uint64[4], device): [0] += solved outputs, [1] += outputs written,
-// [2] += out-of-range actions seen by cube_validate_actions, [3] reserved
+// [2] += out-of-range actions seen by cube_validate_actions, [3] += seeded rows that took the slow path of
+// cube_moves_from_seeds
 namespace cube {
 
 // `last` (n action bytes or null): one more face turn per instance after the `depth` moves (cube_scramble_step)
@@ -45,9 +46,9 @@ int launch_validate(int size, const uint8_t* actions, long long count, unsigned 
                     cudaStream_t stream);
 
 // 2x2x2 leaf expansion (children + parent one-hot, no child one-hot): handles the leading
-// multiple-of-tile parents and returns how many; *rc is 0 or a cudaError_t
+// multiple-of-tile parents and returns how many, or -cudaError
 long long launch_leaf2(const uint8_t* states, long long n, uint8_t* children, void* parent_onehot, int dtype,
-                       uint8_t* solved, float* reward, unsigned long long* counters, cudaStream_t stream, int* rc);
+                       uint8_t* solved, float* reward, unsigned long long* counters, cudaStream_t stream);
 
 // moves[i, :] = np.random.RandomState(seeds[i]).randint(A, size=depth) (cube_env.py:62-65); depth <= 128
 int launch_seeded_moves(int size, const uint32_t* seeds, long long n, int depth, uint8_t* moves,
@@ -58,9 +59,10 @@ int launch_adi_targets(int size, const float* child_values, const uint8_t* child
                        const int* scramble_count, const double* weight, int table_len, long long n,
                        float* target_value, int* target_policy, double* error, cudaStream_t stream);
 
+// the same with the children's one-hot rows (the 2x2x2 ADI shape): leading whole tiles, or -cudaError
 long long launch_leaf2_children(const uint8_t* states, long long n, uint8_t* children, void* child_onehot,
                                 void* parent_onehot, int dtype, uint8_t* solved, float* reward,
-                                unsigned long long* counters, cudaStream_t stream, int* rc);
+                                unsigned long long* counters, cudaStream_t stream);
 
 // batched MCTS (mcts.py:17-154): traverse all trees to their leaves / insert the expanded leaves,
 // back-propagate and test for solved children
@@ -84,12 +86,5 @@ int launch_solve_optimal2(const uint8_t* table, const uint8_t* states, long long
 size_t peer_buffer_bytes(int cap);
 int launch_peer_allreduce_i64(int world, int rank, const uint64_t* peer_bufs, long long* values, int n, int cap,
                               unsigned epoch, cudaStream_t stream);
-
-int sm_count();
-// index of the current device for per-device launch state (cudaFuncSetAttribute is per device), 0..63
-int device_slot();
-// CTAs of a persistent (one-per-SM) grid: sm_count() minus the SMs the caller reserved for other
-// kernels (cube_set_reserved_sms / CUBE_RESERVED_SMS), e.g. one for NCCL's reduction kernel
-int persistent_ctas();
 
 }  // namespace cube

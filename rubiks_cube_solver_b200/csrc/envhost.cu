@@ -11,7 +11,6 @@
 // two kernels, three downloads with their synchronisations) took ~120 us per step; the reference's own NumPy
 // step takes ~25 us on the same host.
 #include <atomic>
-#include <cstdlib>
 #include <cstring>
 #include <cuda_runtime.h>
 #include <new>
@@ -19,6 +18,7 @@
 #include "../../include/cube_b200.h"
 #include "cube_threads.cuh"
 #include "cube_kernels.h"
+#include "cube_launch.cuh"
 
 struct cube_env_host {
     int cube_size, max_depth;
@@ -34,7 +34,7 @@ namespace {
 
 inline int round16(int x) { return (x + 15) & ~15; }
 
-const bool g_spin = !(getenv("CUBE_ENV_SPIN") && getenv("CUBE_ENV_SPIN")[0] == '0');    // A/B switch
+const bool g_spin = cube::env_flag("CUBE_ENV_SPIN", true);     // A/B switch
 
 // One cube: `depth` moves (indices >= A are no-ops, like the batch kernels' identity rows) applied to the row at
 // `in` (or to the solved cube when in == nullptr), then the verdict and the uint8 one-hot rows.  All pointers are

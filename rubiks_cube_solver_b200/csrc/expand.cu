@@ -18,6 +18,7 @@
 #include <cuda_runtime.h>
 #include "cube_threads.cuh"
 #include "cube_kernels.h"
+#include "cube_launch.cuh"
 
 namespace {
 
@@ -287,12 +288,7 @@ int launch_one(const uint8_t* states, long long n, uint8_t* children, void* chil
     // the phases of a tile are separated by barriers, so overlap comes from having many CTAs
     // per SM in different phases, scheduled by the hardware
     const long long grid = n_tiles < 0x7fffffffLL ? n_tiles : 0x7fffffffLL;
-    static bool configured[64] = {};                       // per device: function attributes are per device
-    bool& done = configured[cube::device_slot()];
-    if (!done) {
-        cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        done = true;
-    }
+    cube::prefer_max_shared(kern);
     kern<<<(unsigned)grid, kThreads, 0, stream>>>(states, n, children, (uint8_t*)child_onehot,
                                                   (uint8_t*)parent_onehot, solved, reward, counters, child_codes,
                                                   parent_codes, exact);
@@ -309,39 +305,29 @@ int launch_expand(int size, const uint8_t* states, long long n, uint8_t* childre
 {
     if (n == 0) return 0;
     const int exact = (size == 3 && encoding == CUBE_ENCODING_EXACT) ? 1 : 0;
-    if (size == 2 && child_onehot && dtype != 1) {
-        // 2x2x2 ADI shape: image kernel K3c for whole tiles of parents, generic kernel for the remainder
-        // (f32: the generic kernel already streams at the HBM peak, 1.03 measured; K3c with 8 parents per
-        // CTA reached 0.98)
-        int rc = 0;
-        const long long done = launch_leaf2_children(states, n, children, child_onehot, parent_onehot, dtype, solved,
-                                                     reward, counters, stream, &rc);
-        if (rc) return rc;
-        if (done == n) return 0;
-        const int es = dtype == 0 ? 2 : (dtype == 1 ? 4 : 1);
-        states += done * 24;
+    // 2x2x2: whole tiles of parents through a dedicated kernel, the remainder through the generic kernel below.
+    // The ADI shape takes the image kernel K3c (f32: the generic kernel already streams at the HBM peak, 1.03
+    // measured; K3c with 8 parents per CTA reached 0.98), the MCTS leaf shape (BASELINE config 5) the
+    // register-resident kernel.
+    long long done = 0;
+    if (size == 2 && child_onehot && dtype != 1)
+        done = launch_leaf2_children(states, n, children, child_onehot, parent_onehot, dtype, solved, reward, counters,
+                                     stream);
+    else if (size == 2 && !child_onehot && (children || parent_onehot))
+        done = launch_leaf2(states, n, children, parent_onehot, dtype, solved, reward, counters, stream);
+    if (done < 0) return (int)-done;
+    if (done == n) return 0;
+    if (done > 0) {                                          // the generic kernel takes the parents after the tiles
+        using G = CubeGeom<2>;
+        const long long es = dtype == 0 ? 2 : (dtype == 1 ? 4 : 1);
+        auto skip = [done](auto* p, long long per_parent) { return p ? p + done * per_parent : p; };
+        states += done * G::S;
         n -= done;
-        if (children) children += done * 144;
-        child_onehot = static_cast<uint8_t*>(child_onehot) + done * 6 * 147 * es;
-        if (parent_onehot) parent_onehot = static_cast<uint8_t*>(parent_onehot) + done * 147 * es;
-        if (solved) solved += done * 6;
-        if (reward) reward += done * 6;
-    }
-    if (size == 2 && !child_onehot && (children || parent_onehot)) {
-        // the MCTS leaf shape (BASELINE config 5): register-resident kernel for whole tiles,
-        // the generic kernel below for the ragged remainder
-        int rc = 0;
-        const long long done = launch_leaf2(states, n, children, parent_onehot, dtype, solved, reward, counters,
-                                            stream, &rc);
-        if (rc) return rc;
-        if (done == n) return 0;
-        const int es = dtype == 0 ? 2 : (dtype == 1 ? 4 : 1);
-        states += done * 24;
-        n -= done;
-        if (children) children += done * 144;
-        if (parent_onehot) parent_onehot = static_cast<uint8_t*>(parent_onehot) + done * 147 * es;
-        if (solved) solved += done * 6;
-        if (reward) reward += done * 6;
+        children = skip(children, G::A * G::S);
+        child_onehot = skip(static_cast<uint8_t*>(child_onehot), G::A * G::D * es);
+        parent_onehot = skip(static_cast<uint8_t*>(parent_onehot), G::D * es);
+        solved = skip(solved, G::A);
+        reward = skip(reward, G::A);
     }
 #define CUBE_EXPAND_CASE(SZ, DT)                                                                         \
     if (size == SZ && dtype == DT)                                                                       \

@@ -14,10 +14,10 @@
 // 4 warps per SM, 30 dependent levels per lane: 0.095 ms for config 4's parents, occupancy 6 %.)  Replaces one cube_walk launch
 // per depth level plus the step-major -> cube-major transposes of round 1 (adi.py).
 // HBM traffic per cube: depth (moves in) + depth * (S + 1) bytes out.
-#include <atomic>
 #include <cuda_runtime.h>
 #include "cube_bulk.cuh"
 #include "cube_kernels.h"
+#include "cube_launch.cuh"
 #include "cube_threads.cuh"
 
 namespace {
@@ -25,7 +25,6 @@ namespace {
 constexpr int kSplit = 4;                          // lanes per cube: the levels of a cube are split four ways
 constexpr int kCubesPerTile = 32 / kSplit;
 constexpr int kMaxWarps = 16;
-constexpr int kSmemLimit = 227 * 1024;
 
 template <int SIZE>
 struct PrefixSmem {
@@ -113,18 +112,12 @@ int launch_one(const uint8_t* moves, long long n, int depth, uint8_t* out, uint8
                cudaStream_t stream)
 {
     using L = PrefixSmem<SIZE>;
-    int warps = (kSmemLimit - L::kPerWarp) / L::per_warp(depth);
+    const int warps = cube::warps_that_fit(L::kPerWarp, L::per_warp(depth), kMaxWarps);
     if (warps < 1) return CUBE_ERR_ARG;                                 // depth too large for one tile image
-    if (warps > kMaxWarps) warps = kMaxWarps;
     const int smem = L::bytes(depth, warps);
     auto kern = prefix_kernel<SIZE>;
-    static std::atomic<int> configured_dev[64];                        // per device, 0 = never configured
-    std::atomic<int>& configured = configured_dev[cube::device_slot()];
-    if (smem > configured.load(std::memory_order_relaxed)) {
-        const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return (int)e;
-        configured.store(smem, std::memory_order_relaxed);
-    }
+    const cudaError_t e = cube::raise_smem_limit(kern, smem);
+    if (e != cudaSuccess) return (int)e;
     const long long n_tiles = (n + kCubesPerTile - 1) / kCubesPerTile;
     long long grid = (n_tiles + warps - 1) / warps;
     if (grid > cube::sm_count()) grid = cube::sm_count();
@@ -139,7 +132,7 @@ namespace cube {
 int prefix_max_depth(int size)
 {
     const int per_level = kCubesPerTile * (size == 3 ? 54 : 24) + kCubesPerTile;
-    return (kSmemLimit - (size == 3 ? PrefixSmem<3>::kPerWarp : PrefixSmem<2>::kPerWarp) - 32) / per_level;
+    return (cube::kSmemPerBlock - (size == 3 ? PrefixSmem<3>::kPerWarp : PrefixSmem<2>::kPerWarp) - 32) / per_level;
 }
 
 int launch_prefixes(int size, const uint8_t* moves, long long n, int depth, uint8_t* states_out, uint8_t* solved,

@@ -17,13 +17,12 @@
 // different sector per lane).  Several CTAs per SM overlap load, compute and store.
 // The kernel is bound by the ALU pipe (PRMT/LOP3) and the shared-memory pipe (six
 // table words per move), not by HBM -- see DESIGN.md.
-#include <atomic>
-#include <cstdlib>
 #include <cstring>
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include "cube_bulk.cuh"
 #include "cube_kernels.h"
+#include "cube_launch.cuh"
 #include "cube_sched.cuh"
 #include "cube_threads.cuh"
 
@@ -491,27 +490,19 @@ long long launch_sliced(const uint8_t* moves, long long n, int depth, uint8_t* o
     if (n_tiles < 1) return 0;
     if (n_tiles > 0x3fffffff) n_tiles = 0x3fffffff;
     static const int slice = [] {
-        const char* e = getenv("CUBE_SLICE");
-        const int v = e ? atoi(e) : kSliceDefault;
+        const int v = cube::env_int("CUBE_SLICE", kSliceDefault);
         return (v >= 16 && v <= 240 && v % 16 == 0) ? v : kSliceDefault;
     }();
-    int warps = (227 * 1024 - 256 - L::kFixed) / L::per_warp(slice);
-    if (warps > 8) warps = 8;
+    int warps = cube::warps_that_fit(256 + L::kFixed, L::per_warp(slice), 8);
     if (warps >= 4) warps &= ~3;                                      // the same number on every scheduler
     if (warps < 1) return 0;
     const int smem = L::bytes(warps, slice) + 256 < 66048 + 256 ? 66048 + 256 : L::bytes(warps, slice) + 256;
     auto kern = scramble_sliced_kernel<SIZE>;
-    static std::atomic<int> configured_dev[64];
-    std::atomic<int>& cfg = configured_dev[cube::device_slot()];
-    if (smem > cfg.load(std::memory_order_relaxed)) {
-        const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return -(long long)e;
-        cfg.store(smem, std::memory_order_relaxed);
-    }
-    long long grid = (n_tiles + warps - 1) / warps;
-    if (grid > cube::persistent_ctas()) grid = cube::persistent_ctas();
-    kern<<<(unsigned)grid, warps * 32, smem, stream>>>(moves, (int)n_tiles, depth, out, solved, reward, counters, last, slice);
-    const cudaError_t e = cudaGetLastError();
+    cudaError_t e = cube::raise_smem_limit(kern, smem);
+    if (e != cudaSuccess) return -(long long)e;
+    kern<<<cube::persistent_grid(n_tiles, warps), warps * 32, smem, stream>>>(moves, (int)n_tiles, depth, out, solved, reward,
+                                                                            counters, last, slice);
+    e = cudaGetLastError();
     if (e != cudaSuccess) return -(long long)e;
     return n_tiles * 64;
 }
@@ -578,16 +569,10 @@ int launch_classic(const uint8_t* moves, long long n, int depth, uint8_t* out, u
     if (staged) {
         auto kern_full = scramble_tile_kernel<SIZE, true>;
         auto kern_tail = scramble_tile_kernel<SIZE, false>;
-        static std::atomic<int> configured_dev[64];         // per device, 0 = never configured; host threads may race here
-        std::atomic<int>& configured_smem = configured_dev[cube::device_slot()];
-        if (smem > configured_smem.load(std::memory_order_relaxed)) {
-            cudaError_t e = cudaFuncSetAttribute(kern_full, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-            if (e == cudaSuccess) e = cudaFuncSetAttribute(kern_tail, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-            if (e != cudaSuccess) return (int)e;
-            // largest shared-memory carve-out, so occupancy is set by registers, not by the default split
-            cudaFuncSetAttribute(kern_full, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-            configured_smem.store(smem, std::memory_order_relaxed);
-        }
+        cudaError_t e = cube::raise_smem_limit(kern_full, smem);
+        if (e == cudaSuccess) e = cube::raise_smem_limit(kern_tail, smem);
+        if (e != cudaSuccess) return (int)e;
+        cube::prefer_max_shared(kern_full);
         const long long full_tiles = n / kTile;
         if (full_tiles > 0)
             kern_full<<<(unsigned)full_tiles, kTile, smem, stream>>>(moves, n, 0, depth, out, solved, reward, counters, last);
@@ -604,8 +589,6 @@ int launch_classic(const uint8_t* moves, long long n, int depth, uint8_t* out, u
     }
     return (int)cudaGetLastError();
 }
-
-constexpr int kSmemLimit = 227 * 1024;
 
 // Tensor map of a move array for the swizzled tiles of K1p: the bytes as rows of 128, a box = one tile of
 // 64 / 128 move rows (`tile_rows` = tile * depth / 128 rows of 128 bytes), 128-byte swizzle on the shared-memory side.  The encoder is a
@@ -645,17 +628,15 @@ long long launch_pairs(const uint8_t* moves, long long n, int depth, uint8_t* ou
     constexpr int kPairTile = L::kPairTile;
     if (n < kPairTile) return 0;
     // depths whose flat row stride bank-conflicts on the move words are staged as swizzled tiles
-    static const bool swz_ok = !(getenv("CUBE_PAIR_SWIZZLE") && getenv("CUBE_PAIR_SWIZZLE")[0] == '0');
+    static const bool swz_ok = cube::env_flag("CUBE_PAIR_SWIZZLE", true);
     static_assert(L::kPerWarp % 1024 == 0, "the per-warp areas of the swizzled variant start on 1 KB");
     long long n_tiles = n / kPairTile;
     if (n_tiles > 0x3fffffff) n_tiles = 0x3fffffff;                   // 32-bit tile counters; the caller handles the rest
     const int tile_rows = kPairTile * depth / 128;                    // of the tensor map, when swizzled
     constexpr bool kCanSwizzle = SIZE == 2 || NS == 2;                // 3x3x3 with four instances per lane: flat only
     bool priv = kCanSwizzle && swz_ok && depth % (SIZE == 3 ? 8 : 16) == 0 && n_tiles * tile_rows < 0x7fffffffLL;
-    auto warps_for = [&](bool p) {
-        int w = (kSmemLimit - (p ? 1024 : 256) - L::kPerWarp) / L::per_warp(depth, p);
-        if (w > PairCfg<SIZE, NS>::kMaxWarps) w = PairCfg<SIZE, NS>::kMaxWarps;
-        return w & ~3;                                                // the same number on every scheduler
+    auto warps_for = [&](bool p) {                                    // the same number on every scheduler
+        return cube::warps_that_fit((p ? 1024 : 256) + L::kPerWarp, L::per_warp(depth, p), PairCfg<SIZE, NS>::kMaxWarps) & ~3;
     };
     if (warps_for(priv) < min_warps) return 0;
     alignas(64) CUtensorMap move_map;
@@ -678,31 +659,12 @@ long long launch_pairs(const uint8_t* moves, long long n, int depth, uint8_t* ou
         {scramble_pairs_kernel<SIZE, 0, NS, 1>, scramble_pairs_kernel<SIZE, 30, NS, 1>, scramble_pairs_kernel<SIZE, 20, NS, 1>, scramble_pairs_kernel<SIZE, kSwz, NS, 1>},
         {scramble_pairs_kernel<SIZE, 0, NS, kM2>, scramble_pairs_kernel<SIZE, 30, NS, kM2>, scramble_pairs_kernel<SIZE, 20, NS, kM2>, scramble_pairs_kernel<SIZE, kSwz, NS, kM2>}};
     const Kern kern = kerns[mode][variant];
-    static std::atomic<int> configured_smem[64][12];      // per device and kernel, 0 = never configured
-    std::atomic<int>& cfg = configured_smem[cube::device_slot()][variant + 4 * mode];
-    if (smem > cfg.load(std::memory_order_relaxed)) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        if (e != cudaSuccess) return -(long long)e;
-        cfg.store(smem, std::memory_order_relaxed);
-    }
-    long long grid = (n_tiles + warps - 1) / warps;
-    if (grid > cube::persistent_ctas()) grid = cube::persistent_ctas();
+    cudaError_t e = cube::raise_smem_limit(kern, smem);
+    if (e != cudaSuccess) return -(long long)e;
     sched::Slot* slot = sched::claim_slot();
     if (!slot) return -(long long)cudaErrorUnknown;
-    cudaLaunchConfig_t cfg_l = {};
-    cfg_l.gridDim = dim3((unsigned)grid);
-    cfg_l.blockDim = dim3((unsigned)(warps * 32));
-    cfg_l.dynamicSmemBytes = (size_t)smem;
-    cfg_l.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    static const bool pdl = !(getenv("CUBE_PDL") && getenv("CUBE_PDL")[0] == '0');
-    cfg_l.attrs = attr;
-    cfg_l.numAttrs = pdl ? 1 : 0;
-    cudaError_t e = cudaLaunchKernelEx(&cfg_l, kern, moves, (int)n_tiles, depth, out, solved, reward, counters, slot,
-                                       sched::tail_div(), move_map, last);
-    if (e == cudaSuccess) e = cudaGetLastError();
+    e = cube::launch_pdl(kern, cube::persistent_grid(n_tiles, warps), warps * 32, smem, stream, moves, (int)n_tiles, depth,
+                         out, solved, reward, counters, slot, sched::tail_div(), move_map, last);
     if (e != cudaSuccess) return -(long long)e;
     return n_tiles * kPairTile;
 }
@@ -713,20 +675,20 @@ int launch_one(const uint8_t* moves, long long n, int depth, uint8_t* out, uint8
 {
     using G = CubeGeom<SIZE>;
     long long done = 0;
-    static const char* const force = getenv("CUBE_SCRAMBLE_CLASSIC");               // A/B switch for profiling
-    static const bool four_ok = !(getenv("CUBE_PAIR_FOUR") && getenv("CUBE_PAIR_FOUR")[0] == '0');
+    static const bool classic = cube::env_flag("CUBE_SCRAMBLE_CLASSIC", false);     // A/B switches for profiling
+    static const bool four_ok = cube::env_flag("CUBE_PAIR_FOUR", true);
+    static const bool sliced_ok = cube::env_flag("CUBE_PAIR_SLICED", true);
     // K1p writes the verdicts of rows 2l, 2l+1 as one 16-bit / float2 word: a sliced solved / reward buffer
     // that is not aligned like that takes the byte-wise tile kernel
     const bool aligned = ((reinterpret_cast<uintptr_t>(solved) & 1u) | (reinterpret_cast<uintptr_t>(reward) & 7u) |
                           (reinterpret_cast<uintptr_t>(last) & 1u)) == 0;
-    if (depth >= 1 && depth <= kMaxPairDepth && aligned && !(force && force[0] == '1')) {
+    if (depth >= 1 && depth <= kMaxPairDepth && aligned && !classic) {
         if (SIZE == 2 && four_ok)
             done = launch_pairs<2, 4>(moves, n, depth, out, solved, reward, counters, stream, kMinWarpsFour, last);
         if (done == 0) done = launch_pairs<SIZE, 2>(moves, n, depth, out, solved, reward, counters, stream, 4, last);
         if (done < 0) return (int)-done;
     }
-    static const bool sliced_ok = !(getenv("CUBE_PAIR_SLICED") && getenv("CUBE_PAIR_SLICED")[0] == '0');
-    if (depth > kMaxPairDepth && aligned && sliced_ok && !(force && force[0] == '1')) {
+    if (depth > kMaxPairDepth && aligned && sliced_ok && !classic) {
         done = launch_sliced<SIZE>(moves, n, depth, out, solved, reward, counters, stream, last);
         if (done < 0) return (int)-done;
     }

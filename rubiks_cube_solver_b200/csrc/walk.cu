@@ -13,11 +13,10 @@
 // depth = 1 is `step`; depth > 1 walks several moves without leaving shared
 // memory; depth = 0 with no output is `cube_solved`.
 // HBM traffic per instance: 2*S + depth + 1 + 4 bytes.
-#include <atomic>
-#include <cstdlib>
 #include <cuda_runtime.h>
 #include "cube_bulk.cuh"
 #include "cube_kernels.h"
+#include "cube_launch.cuh"
 #include "cube_sched.cuh"
 #include "cube_threads.cuh"
 
@@ -274,13 +273,7 @@ template <int SIZE>
 int launch_classic(const uint8_t* in, const uint8_t* moves, long long n, int depth, uint8_t* out, uint8_t* solved,
                    float* reward, unsigned long long* counters, cudaStream_t stream)
 {
-    static bool configured_dev[64] = {};                   // per device: function attributes are per device
-    bool& configured = configured_dev[cube::device_slot()];
-    if (!configured) {
-        cudaFuncSetAttribute(walk_tile_kernel<SIZE, true>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                             cudaSharedmemCarveoutMaxShared);
-        configured = true;
-    }
+    cube::prefer_max_shared(walk_tile_kernel<SIZE, true>);
     const long long full_tiles = n / kTile;
     if (full_tiles > 0)
         walk_tile_kernel<SIZE, true><<<(unsigned)full_tiles, kTile, 0, stream>>>(in, moves, n, 0, depth, out, solved,
@@ -298,46 +291,25 @@ int launch_tiles(const uint8_t* in, const uint8_t* moves, long long n, int depth
     using L = WalkSmem<SIZE>;
     using G = CubeGeom<SIZE>;
     long long done = 0;
-    static const char* const force = getenv("CUBE_WALK_CLASSIC");                   // A/B switch for profiling
+    static const bool classic = cube::env_flag("CUBE_WALK_CLASSIC", false);        // A/B switch for profiling
     // K2p stages the move bytes by bulk copies (16-byte aligned source) and writes the verdicts as 32-bit /
     // float2 words; a caller's sliced tensor (actions_all[t] of a [T, N] array, a view into a larger solved /
     // reward buffer) need not be aligned like that: such calls take the byte-wise tile kernel below
     const bool aligned = ((reinterpret_cast<uintptr_t>(moves) & 15u) | (reinterpret_cast<uintptr_t>(solved) & 3u) |
                           (reinterpret_cast<uintptr_t>(reward) & 7u)) == 0;
-    if (depth >= 1 && depth <= kMaxPrivateDepth && out && n >= kRowsPerTile && aligned && !(force && force[0] == '1')) {
-        int warps = (227 * 1024 - L::kPerWarp) / L::per_warp(depth);
-        if (warps > kMaxWalkWarps) warps = kMaxWalkWarps;
-        warps &= ~3;
+    if (depth >= 1 && depth <= kMaxPrivateDepth && out && n >= kRowsPerTile && aligned && !classic) {
+        const int warps = cube::warps_that_fit(L::kPerWarp, L::per_warp(depth), kMaxWalkWarps) & ~3;
         if (warps >= 8) {
             long long n_tiles = n / kRowsPerTile;
             if (n_tiles > 0x3fffffff) n_tiles = 0x3fffffff;
             const int smem = L::bytes(depth, warps);
             auto kern = walk_private_kernel<SIZE>;
-            static std::atomic<int> configured_dev[64];     // per device, 0 = never configured
-            std::atomic<int>& configured_smem = configured_dev[cube::device_slot()];
-            if (smem > configured_smem.load(std::memory_order_relaxed)) {
-                const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-                if (e != cudaSuccess) return (int)e;
-                configured_smem.store(smem, std::memory_order_relaxed);
-            }
-            long long grid = (n_tiles + warps - 1) / warps;
-            if (grid > cube::persistent_ctas()) grid = cube::persistent_ctas();
+            cudaError_t e = cube::raise_smem_limit(kern, smem);
+            if (e != cudaSuccess) return (int)e;
             sched::Slot* slot = sched::claim_slot();
             if (!slot) return (int)cudaErrorUnknown;
-            cudaLaunchConfig_t cfg_l = {};
-            cfg_l.gridDim = dim3((unsigned)grid);
-            cfg_l.blockDim = dim3((unsigned)(warps * 32));
-            cfg_l.dynamicSmemBytes = (size_t)smem;
-            cfg_l.stream = stream;
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            attr[0].val.programmaticStreamSerializationAllowed = 1;
-            static const bool pdl = !(getenv("CUBE_PDL") && getenv("CUBE_PDL")[0] == '0');
-            cfg_l.attrs = attr;
-            cfg_l.numAttrs = pdl ? 1 : 0;
-            cudaError_t e = cudaLaunchKernelEx(&cfg_l, kern, in, moves, (int)n_tiles, depth, out, solved, reward, counters, slot,
-                                               sched::tail_div());
-            if (e == cudaSuccess) e = cudaGetLastError();
+            e = cube::launch_pdl(kern, cube::persistent_grid(n_tiles, warps), warps * 32, smem, stream, in, moves, (int)n_tiles,
+                                 depth, out, solved, reward, counters, slot, sched::tail_div());
             if (e != cudaSuccess) return (int)e;
             done = n_tiles * kRowsPerTile;
         }

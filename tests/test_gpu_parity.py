@@ -1423,10 +1423,27 @@ def test_adi_generate_samples_bf16_passthrough_within_tolerance(size):
     assert np.allclose(a32["error"].cpu().numpy(), err, rtol=0, atol=1e-12)
 
 
-@pytest.mark.parametrize("switch", ["CUBE_PAIR_SWIZZLE=0", "CUBE_PAIR_FOUR=0", "CUBE_SCRAMBLE_CLASSIC=1", "CUBE_TAIL_DIV=1"])
+_SCRAMBLE_K = ("test_scramble_vs_oracle_depths or test_scramble_tile_and_depth_boundaries or "
+               "test_garbage_action_bytes_are_memory_safe_scramble or test_scramble_swizzled_move_tiles")
+_DEEP_K = ("test_deep_scrambles_sliced_kernel or ((test_scramble_vs_oracle_depths or test_scramble_tile_and_depth_boundaries "
+           "or test_garbage_action_bytes_are_memory_safe_scramble) and (321 or 400))")
+_WALK_K = ("test_walk_tile_and_depth_boundaries or test_walk_vs_oracle_any_bytes or "
+           "test_garbage_action_bytes_are_memory_safe_step_and_walk")
+# every A/B switch with the tests that reach the path it controls
+_SWITCH_K = {
+    "CUBE_PAIR_SWIZZLE=0": _SCRAMBLE_K, "CUBE_PAIR_FOUR=0": _SCRAMBLE_K, "CUBE_SCRAMBLE_CLASSIC=1": _SCRAMBLE_K,
+    "CUBE_TAIL_DIV=1": _SCRAMBLE_K, "CUBE_PAIR_SLICED=0": _DEEP_K, "CUBE_SLICE=240": _DEEP_K, "CUBE_WALK_CLASSIC=1": _WALK_K,
+    "CUBE_PDL=0": _SCRAMBLE_K + " or " + _WALK_K, "CUBE_K3C_TILE=32": "test_expand_vs_oracle",
+    "CUBE_K3C_TILE=8": "test_expand_vs_oracle", "CUBE_ENV_SPIN=0": "test_host_cube_single_cube_calls or test_cube_env_drop_in",
+    # 148 SMs - 146: two persistent CTAs, many tiles per warp
+    "CUBE_RESERVED_SMS=146": "test_persistent_kernels_on_concurrent_streams_and_in_a_graph or test_scramble_tile_and_depth_boundaries",
+}
+
+
+@pytest.mark.parametrize("switch", list(_SWITCH_K))
 def test_fallback_paths_under_ab_switches(switch):
     """The library reads its A/B switches (DESIGN.md 7b) once per process, so every fallback path gets its own
-    interpreter: the depth / boundary / garbage-byte scramble tests again, with the switch set.  (The default paths
+    interpreter: the tests that reach the path a switch controls again, with the switch set.  (The default paths
     are what the rest of this file runs; all switches x the whole scramble / step / walk selection were run by hand
     on the final tree, DESIGN.md 7b.)"""
     import subprocess
@@ -1434,12 +1451,114 @@ def test_fallback_paths_under_ab_switches(switch):
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     name, value = switch.split("=")
     env = dict(os.environ, **{name: value})
-    k = ("test_scramble_vs_oracle_depths or test_scramble_tile_and_depth_boundaries or "
-         "test_garbage_action_bytes_are_memory_safe_scramble or test_scramble_swizzled_move_tiles")
+    k = _SWITCH_K[switch]
     out = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_gpu_parity.py"), "-m", "gpu", "-x", "-q",
                           "-p", "no:cacheprovider", "-k", k], capture_output=True, text=True, timeout=600, env=env, cwd=root)
     assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-2000:]
     assert " passed" in out.stdout and " failed" not in out.stdout
+
+
+def test_concurrent_first_use_from_host_threads():
+    """Host threads that make the first calls of a process at the same time: per-device kernel attributes,
+    scheduler slots and switches are set up concurrently (ctypes releases the GIL, so the launchers' host code
+    really overlaps).  Eight threads behind a barrier, each on its own stream, run every launcher in a different
+    order; every output equals the oracle."""
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    script = r'''
+import threading
+import numpy as np
+import torch
+from rubiks_cube_solver_b200 import _lib, ops
+from oracle import cube_np as O
+from oracle import tables as T
+
+_lib.load()                                        # loads the library; no launcher has run yet
+dev = torch.device("cuda", 0)
+rng = np.random.RandomState(23)
+n, n_par, n_threads = 5000, 4099, 8
+
+
+def cu(a):
+    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.uint8)).to(dev)
+
+
+def verdicts(size, st):
+    ok = O.is_solved(size, st)
+    return st, ok, O.rewards(ok)
+
+
+want, calls, step_start = {}, [], {}               # want: the oracle's arrays in the order the call returns them
+for size in (2, 3):
+    A = T.N_ACTIONS[size]
+    for depth in (30, 32, 400):                    # K1p, K1p with swizzled move tiles, sliced K1p
+        m = rng.randint(A, size=(n, depth)).astype(np.uint8)
+        want["scramble%d_%d" % (size, depth)] = verdicts(size, O.scramble(size, m))
+        calls.append(("scramble%d_%d" % (size, depth), lambda st, size=size, m=cu(m): ops.scramble(size, m)))
+    start = O.scramble(size, rng.randint(A, size=(n, 9)))
+    act = rng.randint(A, size=n).astype(np.uint8)
+    step_start[size] = start
+    want["step%d" % size] = verdicts(size, O.apply_moves(size, start, act))
+    calls.append(("step%d" % size, lambda st, size=size, a=cu(act): ops.step(size, st[size], a)))
+    wm = rng.randint(A, size=(n, 5)).astype(np.uint8)
+    want["walk%d" % size] = verdicts(size, O.scramble(size, wm, init=start))
+    calls.append(("walk%d" % size, lambda st, size=size, x=cu(start), m=cu(wm): ops.walk(size, x, m)))
+    par = O.scramble(size, rng.randint(A, size=(n_par, 9)))
+    ch, ok = O.expand(size, par)
+    ch_oh = O.encode(size, ch.reshape(n_par * A, -1)).reshape(n_par, A, *T.STATE_DIM[size])
+    want["adi%d" % size] = (ch, ch_oh, O.encode(size, par), ok, O.rewards(ok))
+    calls.append(("adi%d" % size, lambda st, size=size, p=cu(par): tuple(
+        ops.expand(size, p, want_children=True, want_parent_onehot=True)[k]
+        for k in ("children", "child_onehot", "parent_onehot", "solved", "reward"))))
+    if size == 2:                                  # the MCTS leaf shape
+        want["leaf2"] = (ch, O.encode(2, par), ok, O.rewards(ok))
+        calls.append(("leaf2", lambda st, p=cu(par): tuple(
+            ops.expand(2, p, want_children=True, want_child_onehot=False, want_parent_onehot=True)[k]
+            for k in ("children", "parent_onehot", "solved", "reward"))))
+    pm = rng.randint(A, size=(n, 30)).astype(np.uint8)
+    _, trail, flags = O.scramble(size, pm, per_step=True)
+    want["prefixes%d" % size] = (trail, flags)
+    calls.append(("prefixes%d" % size, lambda st, size=size, m=cu(pm): ops.scramble_prefixes(size, m, want_solved=True)))
+torch.cuda.synchronize()
+
+barrier = threading.Barrier(n_threads)
+results, errors = [None] * n_threads, []
+
+
+def worker(i):
+    try:
+        stream = torch.cuda.Stream(dev)
+        st = {size: cu(step_start[size]) for size in (2, 3)}   # cube_step works in place: one copy per thread
+        torch.cuda.synchronize()
+        order = calls[i * len(calls) // n_threads:] + calls[:i * len(calls) // n_threads]
+        with torch.cuda.stream(stream):
+            barrier.wait()
+            results[i] = {name: fn(st) for name, fn in order}
+        stream.synchronize()
+    except BaseException as e:                     # noqa: BLE001
+        errors.append(repr(e))
+        barrier.abort()
+
+
+threads = [threading.Thread(target=worker, args=(i,)) for i in range(n_threads)]
+for t in threads:
+    t.start()
+for t in threads:
+    t.join()
+assert not errors, errors
+for i, res in enumerate(results):
+    for name, exp in want.items():
+        got = res[name]
+        assert len(got) == len(exp), name
+        for g, w in zip(got, exp):
+            g = g.float().cpu().numpy() if g.dtype == torch.bfloat16 else g.cpu().numpy()
+            assert g.shape == w.shape and (g == w.astype(g.dtype)).all(), (i, name)
+print("checked", len(results), "threads x", len(want), "calls")
+'''
+    out = subprocess.run([sys.executable, "-c", script], capture_output=True, text=True, timeout=600, cwd=root)
+    assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-3000:]
+    assert "checked 8 threads x 15 calls" in out.stdout
 
 
 def test_bench_dump_outputs(tmp_path):
