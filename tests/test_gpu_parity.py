@@ -1429,6 +1429,13 @@ _DEEP_K = ("test_deep_scrambles_sliced_kernel or ((test_scramble_vs_oracle_depth
            "or test_garbage_action_bytes_are_memory_safe_scramble) and (321 or 400))")
 _WALK_K = ("test_walk_tile_and_depth_boundaries or test_walk_vs_oracle_any_bytes or "
            "test_garbage_action_bytes_are_memory_safe_step_and_walk")
+# test_optional_outputs_gpu.py: every output set on the same paths
+_SCRAMBLE_K += (" or test_scramble_every_output_set or test_scramble_output_sets_many_tiles_per_warp or "
+                "test_scramble_partial_flags_unaligned or test_scramble_step_abi_output_sets or "
+                "test_noop_padded_reference_scrambles_without_flags or test_host_pipeline_flag_combinations")
+_DEEP_K += (" or ((test_scramble_every_output_set or test_scramble_partial_flags_unaligned or "
+            "test_scramble_step_abi_output_sets) and (321 or 400))")
+_WALK_K += " or test_walk_and_step_abi_output_sets"
 # every A/B switch with the tests that reach the path it controls
 _SWITCH_K = {
     "CUBE_PAIR_SWIZZLE=0": _SCRAMBLE_K, "CUBE_PAIR_FOUR=0": _SCRAMBLE_K, "CUBE_SCRAMBLE_CLASSIC=1": _SCRAMBLE_K,
@@ -1452,8 +1459,9 @@ def test_fallback_paths_under_ab_switches(switch):
     name, value = switch.split("=")
     env = dict(os.environ, **{name: value})
     k = _SWITCH_K[switch]
-    out = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_gpu_parity.py"), "-m", "gpu", "-x", "-q",
-                          "-p", "no:cacheprovider", "-k", k], capture_output=True, text=True, timeout=600, env=env, cwd=root)
+    files = [os.path.join(root, "tests", f) for f in ("test_gpu_parity.py", "test_optional_outputs_gpu.py")]
+    out = subprocess.run([sys.executable, "-m", "pytest"] + files + ["-m", "gpu", "-x", "-q", "-p", "no:cacheprovider", "-k", k],
+                         capture_output=True, text=True, timeout=600, env=env, cwd=root)
     assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-2000:]
     assert " passed" in out.stdout and " failed" not in out.stdout
 
