@@ -16,7 +16,7 @@
  *   - every pointer is a DEVICE pointer unless the name ends in _host; arrays
  *     are contiguous.  Sticker rows, one-hot buffers and cube_scramble's move
  *     array must start on a 16-byte boundary, float / int32 arrays on their
- *     natural 4 bytes (CUBE_ERR_ALIGN otherwise); action / move bytes of
+ *     natural 4 bytes, float64 arrays on 8 (CUBE_ERR_ALIGN otherwise); action / move bytes of
  *     cube_step / cube_walk and the solved flags may start anywhere (a sliced
  *     buffer that is not 16- / 8- / 4-byte aligned takes a byte-wise kernel).
  *   - calls are asynchronous on `stream` (a cudaStream_t, may be NULL), never
@@ -163,8 +163,10 @@ int cube_solved(int cube_size, const uint8_t* states, int64_t n, uint8_t* solved
 
 /* sim_state_to_state (cube_env.py:132-152): one-hot network input of each row,
  * [n, 20, 24] or [n, 7, 21] elements of `dtype` (bf16 / f32 / u8), exactly one 1
- * per one-hot row; `encoding` = CUBE_ENCODING_REFERENCE (3x3x3 corners through the reference's table as
- * shipped) or CUBE_ENCODING_EXACT. */
+ * per one-hot row for the rows of real states; `encoding` = CUBE_ENCODING_REFERENCE (3x3x3 corners through the
+ * reference's table as shipped) or CUBE_ENCODING_EXACT.  A 2x2x2 row that names a cubelet twice gets what the
+ * reference's loop gives it (cube_env.py:141-147): two 1s in that cubelet's one-hot row, none in the missing
+ * cubelet's. */
 int cube_encode(int cube_size, const uint8_t* states, int64_t n, void* onehot, int dtype, int encoding, void* stream);
 
 /* ADI / MCTS expansion -- the child loop of get_target_value (cube_env.py:212-238)
@@ -250,7 +252,7 @@ int cube_mcts_update(int cube_size, const cube_mcts_tree_t* tree, const uint8_t*
                      int32_t* n_actions, int32_t* n_sims, int32_t* n_active, void* stream);
 
 /* cube_expand with COMPACT CODES instead of the children's one-hot rows: code[row] = the column of the
- * single 1 of that one-hot row (what argmax over the row gives), KEY = (R + 3) & ~3 bytes per state
+ * first 1 of that one-hot row, 0 for a row without a 1 (what argmax over the row gives), KEY = (R + 3) & ~3 bytes per state
  * (8 / 20), zero-padded.  The batched MCTS keys its tree nodes with them (the reference keys its dict with
  * np.array2string of the observation, mcts.py:57,105: equal observations <=> equal codes).
  *   child_codes   [n, A, KEY] uint8  out or NULL

@@ -21,13 +21,15 @@ int fail(int code, const char* what)
         snprintf(t_err, sizeof(t_err), "%s: %s", what,
                  code == CUBE_ERR_SIZE ? "cube_size must be 2 or 3"
                  : code == CUBE_ERR_ARG ? "bad argument (null pointer, negative count or unknown dtype)"
-                 : code == CUBE_ERR_ALIGN ? "device pointers must be 16-byte aligned"
+                 : code == CUBE_ERR_ALIGN ? "misaligned device pointer (sticker, move and one-hot arrays: 16 bytes; "
+                                            "float / int32: 4; float64: 8)"
                  : code == CUBE_ERR_ACTION ? "action index out of range" : "error");
     return code;
 }
 
 inline bool misaligned(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) != 0; }
 inline bool misaligned4(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3u) != 0; }   // float / int32 arrays
+inline bool misaligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7u) != 0; }   // float64 arrays
 
 #define CUBE_CHECK_SIZE(fn) if (cube_size != 2 && cube_size != 3) return fail(CUBE_ERR_SIZE, fn)
 
@@ -166,7 +168,9 @@ int cube_adi_targets(int cube_size, const float* child_values, const uint8_t* ch
     if (n < 0 || table_len < 0 || (n > 0 && (!child_values || !child_solved || !parent_values || !scramble_count ||
                                              !weight || !target_value || !target_policy || !error)))
         return fail(CUBE_ERR_ARG, "cube_adi_targets");
-    if (misaligned(child_values)) return fail(CUBE_ERR_ALIGN, "cube_adi_targets");
+    if (misaligned(child_values) || misaligned4(parent_values) || misaligned4(scramble_count) || misaligned8(weight) ||
+        misaligned4(target_value) || misaligned4(target_policy) || misaligned8(error))
+        return fail(CUBE_ERR_ALIGN, "cube_adi_targets");
     CUBE_DONE("cube_adi_targets", cube::launch_adi_targets(cube_size, child_values, child_solved, parent_values,
                                                            scramble_count, weight, table_len, n, target_value,
                                                            target_policy, error, (cudaStream_t)stream));
@@ -189,7 +193,8 @@ int cube_expand(int cube_size, const uint8_t* states, int64_t n, uint8_t* childr
     CUBE_CHECK_SIZE("cube_expand");
     if (n < 0 || dtype < 0 || dtype > 2 || encoding < 0 || encoding > 1 || (n > 0 && !states))
         return fail(CUBE_ERR_ARG, "cube_expand");
-    if (misaligned(states) || misaligned(children) || misaligned(child_onehot) || misaligned(parent_onehot))
+    if (misaligned(states) || misaligned(children) || misaligned(child_onehot) || misaligned(parent_onehot) ||
+        misaligned4(reward))
         return fail(CUBE_ERR_ALIGN, "cube_expand");
     CUBE_DONE("cube_expand", cube::launch_expand(cube_size, states, n, children, child_onehot, parent_onehot, dtype,
                                                  solved, reward, (unsigned long long*)counters,
@@ -203,7 +208,7 @@ int cube_expand_codes(int cube_size, const uint8_t* states, int64_t n, uint8_t* 
     CUBE_CHECK_SIZE("cube_expand_codes");
     if (n < 0 || dtype < 0 || dtype > 2 || encoding < 0 || encoding > 1 || (n > 0 && !states))
         return fail(CUBE_ERR_ARG, "cube_expand_codes");
-    if (misaligned(states) || misaligned(children) || misaligned(parent_onehot))
+    if (misaligned(states) || misaligned(children) || misaligned(parent_onehot) || misaligned4(reward))
         return fail(CUBE_ERR_ALIGN, "cube_expand_codes");
     CUBE_DONE("cube_expand_codes", cube::launch_expand_codes(cube_size, states, n, children, child_codes, parent_codes,
                                                              parent_onehot, dtype, solved, reward,

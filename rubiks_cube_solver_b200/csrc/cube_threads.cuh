@@ -802,7 +802,9 @@ CUBE_HD void onehot_set(uint32_t* w, int p)
 }
 
 // The 16-byte vector that starts `off` elements into segment `seg` of a stream of one-hot
-// segments of width C; col[s] = position of the 1 in segment s (255 = none).  A vector touches at
+// segments of width C; col[s] = position of the 1 in segment s (255 = none).  One byte per segment
+// holds the one-hot rows of real states; a 2x2x2 row that names a cubelet twice needs two 1s in a
+// segment and is written element by element (onehot2_element).  A vector touches at
 // most two segments (V <= C).  Branch-free: onehot_set ignores positions outside [0, V), and a
 // 255 column always lands outside; col[] must be readable one entry past the last segment.
 template <int DTYPE, int C>
@@ -823,7 +825,8 @@ CUBE_HD void onehot_vector(int v, const uint8_t* col, int n_seg, uint32_t* w)
     onehot_vector_at<DTYPE, C>(seg, e0 - seg * C, col, w);
 }
 
-// column of the 1 for one (row, slot): 3x3x3 returns the column, 2x2x2 returns cubelet | ori << 4
+// column of the 1 for one (row, slot): 3x3x3 returns the column, 2x2x2 returns cubelet | ori << 4 of the
+// cubelet at position `slot` (cubelet <= 6 for every byte content: the table holds no other value)
 template <int SIZE>
 CUBE_HD uint32_t onehot_code(const uint8_t* row, int slot, const uint32_t* s_def, const uint8_t* s_lut0,
                              const uint8_t* s_lut1)
@@ -832,4 +835,25 @@ CUBE_HD uint32_t onehot_code(const uint8_t* row, int slot, const uint32_t* s_def
     const uint32_t a = row[d & 0xffu], b = row[(d >> 8) & 0xffu], c = row[(d >> 16) & 0xffu];
     if (SIZE == 3 && slot >= 8) return s_lut1[(a + 10u * b) & 127u];
     return s_lut0[(a + 2u * b + 10u * c) & 127u];
+}
+
+// 2x2x2 one-hot element (cubelet `cubelet`, column `col`) of a sticker row, the reference's loop read literally
+// (cube_env.py:141-147: state[cubelet][3 * position + ori] = 1 for every position): 1 exactly when position
+// col / 3 holds that cubelet at orientation col % 3.  A row that names a cubelet twice has two 1s in that
+// cubelet's one-hot row and none in the missing cubelet's; a per-cubelet column byte cannot say that.
+CUBE_HD bool onehot2_element(const uint8_t* row, int cubelet, int col, const uint32_t* s_def, const uint8_t* s_lut0)
+{
+    const int pos = col / 3;
+    return onehot_code<2>(row, pos, s_def, s_lut0, s_lut0) == (uint32_t)(cubelet | (col - 3 * pos) << 4);
+}
+
+// 2x2x2: the lowest column set in cubelet `cubelet`'s one-hot row (what argmax gives), 255 for a row without a 1
+CUBE_HD uint32_t onehot2_first_column(const uint8_t* row, int cubelet, const uint32_t* s_def, const uint8_t* s_lut0)
+{
+    uint32_t col = 255u;
+    for (int pos = 6; pos >= 0; --pos) {
+        const uint32_t code = onehot_code<2>(row, pos, s_def, s_lut0, s_lut0);
+        if ((int)(code & 0xfu) == cubelet) col = 3u * pos + (code >> 4);
+    }
+    return col;
 }

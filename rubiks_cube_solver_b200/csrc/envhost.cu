@@ -71,16 +71,17 @@ env_cube_kernel(const uint8_t* in, const uint8_t* moves, int depth, uint8_t* out
     if (solved && t == 0) *solved = stickers_solved<SIZE>(row) ? 1 : 0;
     if (onehot) {
         for (int i = t; i < (int)sizeof(s_oh) / 4; i += 64) reinterpret_cast<uint32_t*>(s_oh)[i] = 0u;
-        if (SIZE == 2 && t < R) s_col[t] = 255;
         __syncthreads();
         if (t < R) {
             const uint32_t code = onehot_code<SIZE>(row, t, (SIZE == 3) ? kHashDef3 : kHashDef2,
                                                     (SIZE == 3) ? kCornerCol3 : kPieceCode2, kEdgeCol3);
             if (SIZE == 3) s_col[t] = (uint8_t)code;
-            else s_col[code & 0xfu] = (uint8_t)(3 * t + (code >> 4));             // cube_env.py:145-147
+            // one 1 per position, as the reference's loop sets it (cube_env.py:145-147): a row that names a cubelet
+            // twice gets two 1s in that cubelet's one-hot row
+            else s_oh[(code & 0xfu) * C + 3 * t + (code >> 4)] = 1;
         }
         __syncthreads();
-        if (t < R && s_col[t] < C) s_oh[t * C + s_col[t]] = 1;
+        if (SIZE == 3 && t < R && s_col[t] < C) s_oh[t * C + s_col[t]] = 1;
         __syncthreads();
         for (int i = t; i < D / 16; i += 64) reinterpret_cast<int4*>(onehot)[i] = reinterpret_cast<const int4*>(s_oh)[i];
         for (int i = (D / 16) * 16 + t; i < D; i += 64) onehot[i] = s_oh[i];

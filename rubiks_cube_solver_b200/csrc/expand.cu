@@ -14,6 +14,9 @@
 // shared memory, every (row, slot) hash is reduced to one byte (the column of
 // the single 1), and then all threads emit the one-hot rows as fully coalesced
 // 16-byte streaming stores, deciding per vector which of its elements is 1.
+// A 2x2x2 row that names a cubelet twice (no real state does) has two 1s in
+// that cubelet's one-hot row (cube_env.py:141-147), which one byte cannot hold:
+// a tile with such a row writes its one-hot rows element by element instead.
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include "cube_threads.cuh"
@@ -49,6 +52,40 @@ __device__ __forceinline__ void emit_onehot(uint8_t* __restrict__ dst, const uin
         off += kOffStep;
         if (off >= C) { off -= C; ++seg; }
     }
+}
+
+// Element-wise one-hot rows: a ragged last tile, and (2x2x2, `literal`) a tile in which some row names a
+// cubelet twice -- there every element is decided from the row's stickers (`rows`, S bytes per row) the way the
+// reference's loop sets it, not from the column bytes.
+template <int SIZE, int DTYPE>
+__device__ __forceinline__ void emit_onehot_elements(uint8_t* __restrict__ dst, const uint8_t* col, int n_rows,
+                                                     const uint8_t* rows, bool literal, const uint32_t* s_def,
+                                                     const uint8_t* s_lut0, int tid)
+{
+    using G = CubeGeom<SIZE>;
+    constexpr int C = G::C;
+    for (int e = tid; e < n_rows * G::D; e += kThreads) {
+        const int seg = e / C, off = e - seg * C;
+        bool one = col[seg] == off;
+        if (SIZE == 2 && literal) {
+            const int r = seg / G::R;
+            one = onehot2_element(rows + r * G::S, seg - r * G::R, off, s_def, s_lut0);
+        }
+        if (DTYPE == 0) reinterpret_cast<uint16_t*>(dst)[e] = one ? 0x3f80 : 0;
+        else if (DTYPE == 1) reinterpret_cast<uint32_t*>(dst)[e] = one ? 0x3f800000u : 0u;
+        else dst[e] = one ? 1 : 0;
+    }
+}
+
+// 2x2x2: seven positions hold seven cubelets, so a row names a cubelet twice exactly when another cubelet's
+// column byte is still 255 after the column pass.  CTA-wide (a barrier): does any of the first n0 bytes of
+// col0 or n1 bytes of col1 say so?
+__device__ __forceinline__ bool any_unset_column(const uint8_t* col0, int n0, const uint8_t* col1, int n1, int tid)
+{
+    bool unset = false;
+    for (int i = tid; i < n0; i += kThreads) unset |= col0[i] == 255;
+    for (int i = tid; i < n1; i += kThreads) unset |= col1[i] == 255;
+    return __syncthreads_or(unset) != 0;
 }
 
 template <int SIZE, int DTYPE>
@@ -154,6 +191,23 @@ expand_kernel(const uint8_t* __restrict__ states, long long n, uint8_t* __restri
         }
         __syncthreads();
 
+        // 2x2x2 rows that name a cubelet twice: the one-hot rows go element-wise, and the racing column pass
+        // left either of two columns, so the codes are recomputed as the lowest column set
+        bool literal = false;
+        if (SIZE == 2 && (child_onehot || parent_onehot || child_codes || parent_codes)) {
+            literal = any_unset_column(s_colc, need_children ? rows * R : 0, s_colp, need_parent_cols ? cnt * R : 0, tid);
+            if (literal && (child_codes || parent_codes)) {
+                for (int it = tid; it < n_items * R; it += kThreads) {
+                    const int r = it / R, cubelet = it - r * R;
+                    const bool is_child = need_children && r < rows;
+                    const int rr = is_child ? r : r - (need_children ? rows : 0);
+                    const uint8_t* row = is_child ? s_child + rr * S : s_par + rr * S;
+                    (is_child ? s_colc : s_colp)[rr * R + cubelet] = (uint8_t)onehot2_first_column(row, cubelet, s_def, s_lut[0]);
+                }
+                __syncthreads();
+            }
+        }
+
         if (children) {
             const long long byte0 = base * A * S;          // multiple of 16 (kParents = 16)
             const int nbytes = rows * S;
@@ -162,7 +216,7 @@ expand_kernel(const uint8_t* __restrict__ states, long long n, uint8_t* __restri
             for (int i = tid; i < nvec; i += kThreads) __stcs(dst + i, reinterpret_cast<const int4*>(s_child)[i]);
             for (int i = (nvec << 4) + tid; i < nbytes; i += kThreads) children[byte0 + i] = s_child[i];
         }
-        // compact codes: the column of the single 1 of every one-hot row (what argmax over the row gives; a
+        // compact codes: the column of the first 1 of every one-hot row (what argmax over the row gives; a
         // 2x2x2 row without a 1 reads 0 like argmax), KEY bytes per state
         if (child_codes) {
             uint8_t* dst = child_codes + base * A * KEY;
@@ -182,31 +236,17 @@ expand_kernel(const uint8_t* __restrict__ states, long long n, uint8_t* __restri
         }
         if (child_onehot) {
             uint8_t* dst = child_onehot + base * A * (long long)(G::D * ESIZE);
-            if ((rows * G::D * ESIZE) % 16 == 0) {
+            if ((rows * G::D * ESIZE) % 16 == 0 && !literal)
                 emit_onehot<DTYPE, C>(dst, s_colc, rows * R, tid);
-            } else {                                        // ragged last tile: element-wise
-                for (int e = tid; e < rows * G::D; e += kThreads) {
-                    const int seg = e / C, off = e - seg * C;
-                    const bool one = s_colc[seg] == off;
-                    if (DTYPE == 0) reinterpret_cast<uint16_t*>(dst)[e] = one ? 0x3f80 : 0;
-                    else if (DTYPE == 1) reinterpret_cast<uint32_t*>(dst)[e] = one ? 0x3f800000u : 0u;
-                    else dst[e] = one ? 1 : 0;
-                }
-            }
+            else
+                emit_onehot_elements<SIZE, DTYPE>(dst, s_colc, rows, s_child, literal, s_def, s_lut[0], tid);
         }
         if (parent_onehot) {
             uint8_t* dst = parent_onehot + base * (long long)(G::D * ESIZE);
-            if ((cnt * G::D * ESIZE) % 16 == 0) {
+            if ((cnt * G::D * ESIZE) % 16 == 0 && !literal)
                 emit_onehot<DTYPE, C>(dst, s_colp, cnt * R, tid);
-            } else {
-                for (int e = tid; e < cnt * G::D; e += kThreads) {
-                    const int seg = e / C, off = e - seg * C;
-                    const bool one = s_colp[seg] == off;
-                    if (DTYPE == 0) reinterpret_cast<uint16_t*>(dst)[e] = one ? 0x3f80 : 0;
-                    else if (DTYPE == 1) reinterpret_cast<uint32_t*>(dst)[e] = one ? 0x3f800000u : 0u;
-                    else dst[e] = one ? 1 : 0;
-                }
-            }
+            else
+                emit_onehot_elements<SIZE, DTYPE>(dst, s_colp, cnt, s_par, literal, s_def, s_lut[0], tid);
         }
     }
     __syncthreads();
@@ -256,18 +296,12 @@ encode_kernel(const uint8_t* __restrict__ states, long long n, uint8_t* __restri
         else s_col[r * R + (code & 0xfu)] = (uint8_t)(3 * slot + (code >> 4));
     }
     __syncthreads();
+    const bool literal = SIZE == 2 && any_unset_column(s_col, cnt * R, s_col, 0, tid);   // a row names a cubelet twice
     uint8_t* dst = onehot + base * (long long)(G::D * ESIZE);
-    if ((cnt * G::D * ESIZE) % 16 == 0) {
+    if ((cnt * G::D * ESIZE) % 16 == 0 && !literal)
         emit_onehot<DTYPE, C>(dst, s_col, cnt * R, tid);
-    } else {
-        for (int e = tid; e < cnt * G::D; e += kThreads) {
-            const int seg = e / C, off = e - seg * C;
-            const bool one = s_col[seg] == off;
-            if (DTYPE == 0) reinterpret_cast<uint16_t*>(dst)[e] = one ? 0x3f80 : 0;
-            else if (DTYPE == 1) reinterpret_cast<uint32_t*>(dst)[e] = one ? 0x3f800000u : 0u;
-            else dst[e] = one ? 1 : 0;
-        }
-    }
+    else
+        emit_onehot_elements<SIZE, DTYPE>(dst, s_col, cnt, s_rows, literal, s_def, s_lut[0], tid);
 }
 
 template <int SIZE, int DTYPE>

@@ -256,13 +256,18 @@ void expand_t(const uint8_t* states, long long n, uint8_t* children, uint8_t* ch
         }
         for (int r = 0; r < rows; ++r) solved[base * A + r] = stickers_solved<SIZE>(&s_child[r * S]);
         if (children) std::memcpy(children + base * A * S, s_child.data(), (size_t)rows * S);
+        // 2x2x2: a column byte left at 255 means some row names a cubelet twice (any_unset_column of expand.cu)
+        bool literal = false;
+        for (int i = 0; SIZE == 2 && i < rows * R; ++i) literal |= colc[i] == 255;
+        for (int i = 0; SIZE == 2 && i < cnt * R; ++i) literal |= colp[i] == 255;
         for (int pass = 0; pass < 2; ++pass) {
             uint8_t* dst = pass == 0 ? child_oh : parent_oh;
             if (!dst) continue;
             const int nr = pass == 0 ? rows : cnt;
             const uint8_t* col = pass == 0 ? colc.data() : colp.data();
+            const uint8_t* src = pass == 0 ? s_child.data() : s_par;
             dst += base * (pass == 0 ? A : 1) * (long long)(G::D * ES);
-            if ((nr * G::D * ES) % 16 == 0) {
+            if ((nr * G::D * ES) % 16 == 0 && !literal) {
                 const int n_vec = nr * R * C / OneHot<DTYPE>::V;
                 for (int v = 0; v < n_vec; ++v) {
                     uint32_t w[4];
@@ -271,7 +276,10 @@ void expand_t(const uint8_t* states, long long n, uint8_t* children, uint8_t* ch
                 }
             } else {
                 for (int e = 0; e < nr * G::D; ++e) {
-                    const bool one = col[e / C] == e % C;
+                    const int seg = e / C;
+                    const bool one = (SIZE == 2 && literal)
+                                         ? onehot2_element(src + (seg / R) * S, seg % R, e % C, def, lut0)
+                                         : col[seg] == e % C;
                     if (DTYPE == 0) reinterpret_cast<uint16_t*>(dst)[e] = one ? 0x3f80 : 0;
                     else if (DTYPE == 1) reinterpret_cast<uint32_t*>(dst)[e] = one ? 0x3f800000u : 0u;
                     else dst[e] = one ? 1 : 0;

@@ -67,6 +67,28 @@ def test_argument_errors_without_cuda(lib):
         _lib.check(_lib.CUBE_ERR_ALIGN, "x")
 
 
+def test_float_arrays_alignment_without_cuda(lib):
+    """Float and int32 arrays start on 4 bytes and float64 arrays on 8 (include/cube_b200.h), else CUBE_ERR_ALIGN
+    before any launch -- on the device such a pointer would be a misaligned access."""
+    buf = (ctypes.c_uint8 * 256)()
+    base = (ctypes.addressof(buf) + 15) & ~15
+    a = ctypes.c_void_p(base)
+    off = lambda k: ctypes.c_void_p(base + k)
+    for size in (2, 3):
+        for k in (1, 2):
+            assert lib.cube_expand(size, a, 1, None, None, None, 0, 0, None, off(k), None, None) == _lib.CUBE_ERR_ALIGN
+            assert lib.cube_expand_codes(size, a, 1, None, a, None, None, 0, 0, None, off(k), None, None) == _lib.CUBE_ERR_ALIGN
+            assert lib.cube_solved(size, a, 1, None, off(k), None, None) == _lib.CUBE_ERR_ALIGN
+        # cube_adi_targets(size, child_values, child_solved, parent_values, scramble_count, weight, table_len, n,
+        #                  target_value, target_policy, error, stream): one pointer off at a time
+        for i, ks in ((3, (1, 2)), (4, (1, 2)), (5, (1, 4)), (8, (1, 2)), (9, (1, 2)), (10, (1, 4))):
+            for k in ks:
+                args = [size, a, a, a, a, a, 8, 1, a, a, a, None]
+                args[i] = off(k)
+                assert lib.cube_adi_targets(*args) == _lib.CUBE_ERR_ALIGN, (i, k)
+    assert b"float64" in lib.cube_last_error()
+
+
 def test_generated_cuda_tables_are_current():
     subprocess.check_call([sys.executable, os.path.join(ROOT, "rubiks_cube_solver_b200", "csrc", "gen_tables.py"),
                            "--check"])

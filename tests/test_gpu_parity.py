@@ -1437,11 +1437,12 @@ _DEEP_K += (" or ((test_scramble_every_output_set or test_scramble_partial_flags
             "test_scramble_step_abi_output_sets) and (321 or 400))")
 _WALK_K += " or test_walk_and_step_abi_output_sets"
 # every A/B switch with the tests that reach the path it controls
+# K3c (leaf_children_kernel) runs with the children's one-hot rows in bf16 / u8
+_K3C_K = "test_expand_vs_oracle or test_expand_every_output_set or test_expand_rows_that_name_a_cubelet_twice"
 _SWITCH_K = {
     "CUBE_PAIR_SWIZZLE=0": _SCRAMBLE_K, "CUBE_PAIR_FOUR=0": _SCRAMBLE_K, "CUBE_SCRAMBLE_CLASSIC=1": _SCRAMBLE_K,
     "CUBE_TAIL_DIV=1": _SCRAMBLE_K, "CUBE_PAIR_SLICED=0": _DEEP_K, "CUBE_SLICE=240": _DEEP_K, "CUBE_WALK_CLASSIC=1": _WALK_K,
-    "CUBE_PDL=0": _SCRAMBLE_K + " or " + _WALK_K, "CUBE_K3C_TILE=32": "test_expand_vs_oracle",
-    "CUBE_K3C_TILE=8": "test_expand_vs_oracle", "CUBE_ENV_SPIN=0": "test_host_cube_single_cube_calls or test_cube_env_drop_in",
+    "CUBE_PDL=0": _SCRAMBLE_K + " or " + _WALK_K, "CUBE_K3C_TILE=32": _K3C_K, "CUBE_K3C_TILE=8": _K3C_K, "CUBE_ENV_SPIN=0": "test_host_cube_single_cube_calls or test_cube_env_drop_in",
     # 148 SMs - 146: two persistent CTAs, many tiles per warp
     "CUBE_RESERVED_SMS=146": "test_persistent_kernels_on_concurrent_streams_and_in_a_graph or test_scramble_tile_and_depth_boundaries",
 }
@@ -1459,7 +1460,8 @@ def test_fallback_paths_under_ab_switches(switch):
     name, value = switch.split("=")
     env = dict(os.environ, **{name: value})
     k = _SWITCH_K[switch]
-    files = [os.path.join(root, "tests", f) for f in ("test_gpu_parity.py", "test_optional_outputs_gpu.py")]
+    files = [os.path.join(root, "tests", f) for f in ("test_gpu_parity.py", "test_optional_outputs_gpu.py",
+                                                      "test_expand_outputs_gpu.py")]
     out = subprocess.run([sys.executable, "-m", "pytest"] + files + ["-m", "gpu", "-x", "-q", "-p", "no:cacheprovider", "-k", k],
                          capture_output=True, text=True, timeout=600, env=env, cwd=root)
     assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-2000:]

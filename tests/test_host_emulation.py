@@ -5,6 +5,7 @@ import ctypes
 import os
 import re
 import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -202,6 +203,111 @@ def test_expand_emulation(emul, size, dtype, n):
     want_poh = O.encode(size, parents).reshape(n, D).astype(view) * one
     assert (coh.view(view).reshape(n, A, D) == want_coh).all()
     assert (poh.view(view).reshape(n, D) == want_poh).all()
+
+
+def twin_rows(size, n, seed):
+    """Sticker rows the reference encodes but no turn sequence reaches: a random scramble in which one cubie's
+    stickers are copied onto another cubie position -- as they are, or turned (3x3x3 edges also flipped) -- so the
+    row names one piece twice and leaves another out.  Only rows the reference's table lookup accepts are kept
+    (O.encode raises IndexError on a hash outside its table)."""
+    rng = np.random.RandomState(seed)
+    A = T.N_ACTIONS[size]
+    rows = []
+    while len(rows) < n:
+        row = O.scramble(size, rng.randint(A, size=(1, 9)))[0]
+        groups = [T.PIECE_DEFS_2] if size == 2 else [T.CORNER_DEFS_3, T.EDGE_DEFS_3]
+        defs = groups[rng.randint(len(groups))]
+        src, dst = rng.choice(len(defs), 2, replace=False)
+        row[defs[dst]] = np.roll(row[defs[src]], rng.randint(defs.shape[1]))
+        try:
+            O.encode(size, row[None])
+        except IndexError:
+            continue
+        rows.append(row)
+    return np.stack(rows)
+
+
+def _expand_emulation_vs_oracle(emul, size, dtype, parents):
+    n = parents.shape[0]
+    A, S, D = T.N_ACTIONS[size], T.N_STICKERS[size], T.ONEHOT_WIDTH[size]
+    es = (2, 4, 1)[dtype]
+    children = np.empty((n, A, S), dtype=np.uint8)
+    coh = np.empty((n, A, D * es), dtype=np.uint8)
+    poh = np.empty((n, D * es), dtype=np.uint8)
+    solved = np.empty((n, A), dtype=np.uint8)
+    emul.emul_expand(size, dtype, _p(parents), n, _p(children), _p(coh), _p(poh), _p(solved))
+    want_c, want_s = O.expand(size, parents)
+    assert (children == want_c).all() and (solved.astype(bool) == want_s).all()
+    one = {0: np.uint16(0x3f80), 1: np.float32(1.0), 2: np.uint8(1)}[dtype]
+    view = {0: np.uint16, 1: np.float32, 2: np.uint8}[dtype]
+    want_coh = O.encode(size, want_c.reshape(n * A, S)).reshape(n, A, D).astype(view) * one
+    want_poh = O.encode(size, parents).reshape(n, D).astype(view) * one
+    assert (coh.view(view).reshape(n, A, D) == want_coh).all()
+    assert (poh.view(view).reshape(n, D) == want_poh).all()
+
+
+@pytest.mark.parametrize("size", (2, 3))
+@pytest.mark.parametrize("dtype", (0, 1, 2))
+@pytest.mark.parametrize("n", (5, 37, 64, 128))
+def test_expand_emulation_rows_that_name_a_piece_twice(emul, size, dtype, n):
+    """Rows that name a cubie twice among reachable rows, in whole and ragged tiles.  2x2x2: the reference's loop
+    (cube_env.py:141-147) sets one 1 per position, so the twice-named cubelet's one-hot row has two 1s and the
+    missing cubelet's none -- a tile with such a row takes the element-wise path.  3x3x3 writes one column per
+    slot and is unaffected; this pins it."""
+    rng = np.random.RandomState(100 * size + n + dtype)
+    parents = O.scramble(size, rng.randint(T.N_ACTIONS[size], size=(n, 6)))
+    at = sorted({0, n // 2, n - 1})
+    parents[at] = twin_rows(size, len(at), seed=n + dtype)
+    if size == 2:
+        assert (O.encode(2, parents[at]).sum(axis=2) == 2).any(axis=1).all()        # the case under test
+    _expand_emulation_vs_oracle(emul, size, dtype, parents)
+
+
+_ARBITRARY_BYTES_SCRIPT = r"""
+import ctypes, sys
+import numpy as np
+sys.path.insert(0, sys.argv[2])
+from oracle import tables as T
+lib = ctypes.CDLL(sys.argv[1])
+vp, ll = ctypes.c_void_p, ctypes.c_longlong
+lib.emul_expand.argtypes = [ctypes.c_int, ctypes.c_int, vp, ll, vp, vp, vp, vp]
+p = lambda a: a.ctypes.data_as(vp)
+rng = np.random.RandomState(5)
+for size in (2, 3):
+    A, S, D = T.N_ACTIONS[size], T.N_STICKERS[size], T.ONEHOT_WIDTH[size]
+    for dtype, es, one in ((0, 2, 0x3f80), (1, 4, 0x3f800000), (2, 1, 1)):
+        for n in (37, 64, 129):
+            parents = rng.randint(0, 256, size=(n, S)).astype(np.uint8)
+            parents[::3] = rng.randint(0, 8, size=parents[::3].shape)
+            children = np.empty((n, A, S), dtype=np.uint8)
+            coh = np.empty((n, A, D * es), dtype=np.uint8)
+            poh = np.empty((n, D * es), dtype=np.uint8)
+            solved = np.empty((n, A), dtype=np.uint8)
+            lib.emul_expand(size, dtype, p(parents), n, p(children), p(coh), p(poh), p(solved))
+            assert (children == parents[:, T.MOVE_DEFS[size]]).all()
+            assert set(np.unique(solved)) <= {0, 1}
+            view = {0: np.uint16, 1: np.uint32, 2: np.uint8}[dtype]
+            for oh in (coh, poh):
+                assert set(np.unique(oh.view(view))) <= {0, one}, (size, dtype, n)
+print("ok")
+"""
+
+
+def test_expand_emulation_arbitrary_bytes_under_address_sanitizer(tmp_path):
+    """Colour bytes >= 6 (and any other byte) are outside the reference's domain but must stay memory-safe: every
+    table index is masked.  The emulation built with AddressSanitizer and libstdc++ assertions runs such rows
+    through every size and dtype, in whole and ragged tiles: no out-of-range access, one-hot elements 0 or 1,
+    flags 0 or 1, children still the plain gather."""
+    lib = str(tmp_path / "libcube_emul_asan.so")
+    rt = subprocess.run(["g++", "-print-file-name=libasan.so"], capture_output=True, text=True).stdout.strip()
+    if not os.path.isabs(rt) or not os.path.exists(rt):
+        pytest.skip("g++ has no AddressSanitizer runtime")
+    subprocess.check_call(["g++", "-O1", "-g", "-std=c++17", "-shared", "-fPIC", "-w", "-fsanitize=address",
+                           "-fno-omit-frame-pointer", "-D_GLIBCXX_ASSERTIONS", "-o", lib, SRC])
+    env = dict(os.environ, LD_PRELOAD=rt, ASAN_OPTIONS="detect_leaks=0:abort_on_error=0")
+    out = subprocess.run([sys.executable, "-c", _ARBITRARY_BYTES_SCRIPT, lib, os.path.dirname(HERE)], capture_output=True,
+                         text=True, timeout=300, env=env)
+    assert out.returncode == 0 and out.stdout.strip().endswith("ok"), out.stdout[-2000:] + out.stderr[-4000:]
 
 
 def _gen_tables():
