@@ -203,7 +203,16 @@ int cube_adi_targets(int cube_size, const float* child_values, const uint8_t* ch
  * one node: n_slots = numMCTSSim + 1 <= 255).  A node is children_and_data[key] of the reference
  * (mcts.py:103-110): key = the observation, here the one-hot rows' column indices (KEY = 20 bytes for
  * 3x3x3, 8 for 2x2x2: 7 indices + one zero byte), children keys, P, W, N, L and done flags.  All
- * members are DEVICE pointers owned by the caller; A = 12 / 6, S = 54 / 24. */
+ * members are DEVICE pointers owned by the caller; A = 12 / 6, S = 54 / 24.
+ * When n_trees > 0, every pointer except sim_counter must be non-NULL (else CUBE_ERR_ARG), and the kernels'
+ * vector loads need (else CUBE_ERR_ALIGN; both checked before any launch):
+ *   P, W, N, L                                      16 bytes (3x3x3: 48-byte rows) / 8 bytes (2x2x2: 24-byte rows)
+ *   child_slot                                      2 bytes
+ *   node_key, child_key, root_key, root_state,
+ *   leaf_state, path_node, path_action              4 bytes (read and written as 32-bit words)
+ *   n_nodes, rand_ptr, path_len, flags, sim_counter 4 bytes
+ * The same holds for cube_mcts_update's leaf_key and child_key_new (4 bytes) and its value, policy, n_actions,
+ * n_sims and n_active (4 bytes; only n_active may be NULL). */
 typedef struct cube_mcts_tree {
     int32_t n_trees, n_slots, path_cap, rand_cap; /* B, M, capacity of one traversal path, draws per tree */
     uint8_t* node_key;                    /* [B, M, KEY]     key of every expanded node                  */

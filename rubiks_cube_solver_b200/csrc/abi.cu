@@ -1,6 +1,7 @@
 // extern "C" boundary of libcube_b200.so: argument checks, then the launchers.
 // See include/cube_b200.h for the contract of every entry point.
 #include <cstdio>
+#include <initializer_list>
 #include <cuda_runtime.h>
 
 #include "../../include/cube_b200.h"
@@ -22,7 +23,7 @@ int fail(int code, const char* what)
                  code == CUBE_ERR_SIZE ? "cube_size must be 2 or 3"
                  : code == CUBE_ERR_ARG ? "bad argument (null pointer, negative count or unknown dtype)"
                  : code == CUBE_ERR_ALIGN ? "misaligned device pointer (sticker, move and one-hot arrays: 16 bytes; "
-                                            "float / int32: 4; float64: 8)"
+                                            "float / int32: 4; float64: 8; MCTS tree store: see cube_mcts_tree_t)"
                  : code == CUBE_ERR_ACTION ? "action index out of range" : "error");
     return code;
 }
@@ -40,6 +41,29 @@ int fail_distance_size(const char* what)
     return CUBE_ERR_SIZE;
 }
 #define CUBE_DONE(fn, rc) do { int rc_ = (rc); return rc_ ? fail(rc_, fn) : 0; } while (0)
+
+// the tree store of cube_mcts_traverse / cube_mcts_update (include/cube_b200.h): CUBE_ERR_ARG for bad sizes and, with
+// trees, for any NULL pointer but sim_counter; CUBE_ERR_ALIGN for a pointer the kernels load as a vector or a word
+int mcts_tree_check(int cube_size, const cube_mcts_tree_t* t)
+{
+    if (!t || t->n_trees < 0 || t->n_slots < 1 || t->n_slots > 255 || t->path_cap < 1 || t->rand_cap < 1)
+        return CUBE_ERR_ARG;
+    if (t->n_trees == 0) return CUBE_OK;
+    if (!t->node_key || !t->child_key || !t->child_done || !t->P || !t->W || !t->N || !t->L || !t->n_nodes ||
+        !t->active || !t->root_state || !t->root_key || !t->rand_table || !t->rand_ptr || !t->path_node ||
+        !t->path_action || !t->path_len || !t->leaf_state || !t->flags || !t->child_slot)
+        return CUBE_ERR_ARG;
+    const uintptr_t row = cube_size == 3 ? 15u : 7u;                  // int4 / int2 rows of N, P, W, L
+    for (const void* p : {(const void*)t->P, (const void*)t->W, (const void*)t->N, (const void*)t->L})
+        if (reinterpret_cast<uintptr_t>(p) & row) return CUBE_ERR_ALIGN;
+    if (reinterpret_cast<uintptr_t>(t->child_slot) & 1u) return CUBE_ERR_ALIGN;
+    for (const void* p : {(const void*)t->node_key, (const void*)t->child_key, (const void*)t->root_key,
+                          (const void*)t->root_state, (const void*)t->leaf_state, (const void*)t->path_node,
+                          (const void*)t->path_action, (const void*)t->n_nodes, (const void*)t->rand_ptr,
+                          (const void*)t->path_len, (const void*)t->flags, (const void*)t->sim_counter})
+        if (misaligned4(p)) return CUBE_ERR_ALIGN;
+    return CUBE_OK;
+}
 
 }  // namespace
 
@@ -140,9 +164,7 @@ int cube_moves_from_seeds(int cube_size, const uint32_t* seeds, int64_t n, int d
 int cube_mcts_traverse(int cube_size, const cube_mcts_tree_t* tree, float cpuct, int virtual_loss, void* stream)
 {
     CUBE_CHECK_SIZE("cube_mcts_traverse");
-    if (!tree || tree->n_trees < 0 || tree->n_slots < 1 || tree->n_slots > 255 || tree->path_cap < 1 || tree->rand_cap < 1 ||
-        (tree->n_trees > 0 && !tree->child_slot))
-        return fail(CUBE_ERR_ARG, "cube_mcts_traverse");
+    if (const int rc = mcts_tree_check(cube_size, tree)) return fail(rc, "cube_mcts_traverse");
     CUBE_DONE("cube_mcts_traverse", cube::launch_mcts_traverse(cube_size, *tree, cpuct, virtual_loss, (cudaStream_t)stream));
 }
 
@@ -151,10 +173,13 @@ int cube_mcts_update(int cube_size, const cube_mcts_tree_t* tree, const uint8_t*
                      int sim_index, int8_t* actions_out, int32_t* n_actions, int32_t* n_sims, int32_t* n_active, void* stream)
 {
     CUBE_CHECK_SIZE("cube_mcts_update");
-    if (!tree || tree->n_trees < 0 || tree->n_slots < 1 || tree->n_slots > 255 || tree->path_cap < 1 || tree->rand_cap < 1 ||
-        (tree->n_trees > 0 && (!leaf_key || !child_key_new || !child_done_new || !value || !policy || !actions_out ||
-                               !n_actions || !n_sims || !tree->child_slot)))
+    if (const int rc = mcts_tree_check(cube_size, tree)) return fail(rc, "cube_mcts_update");
+    if (tree->n_trees > 0 && (!leaf_key || !child_key_new || !child_done_new || !value || !policy || !actions_out ||
+                              !n_actions || !n_sims))
         return fail(CUBE_ERR_ARG, "cube_mcts_update");
+    if (misaligned4(leaf_key) || misaligned4(child_key_new) || misaligned4(value) || misaligned4(policy) ||
+        misaligned4(n_actions) || misaligned4(n_sims) || misaligned4(n_active))
+        return fail(CUBE_ERR_ALIGN, "cube_mcts_update");
     CUBE_DONE("cube_mcts_update", cube::launch_mcts_update(cube_size, *tree, leaf_key, child_key_new, child_done_new, value,
                                                            policy, value_min, sim_index, actions_out, n_actions, n_sims, n_active,
                                                            (cudaStream_t)stream));

@@ -89,6 +89,70 @@ def test_float_arrays_alignment_without_cuda(lib):
     assert b"float64" in lib.cube_last_error()
 
 
+def test_mcts_tree_pointers_without_cuda(lib):
+    """cube_mcts_traverse / cube_mcts_update check every pointer the kernels dereference before any launch
+    (include/cube_b200.h): NULL -> CUBE_ERR_ARG (only sim_counter and n_active may be NULL), and a pointer the
+    kernels read as a vector or a word off its boundary -> CUBE_ERR_ALIGN.  Every case here is rejected, so
+    nothing reaches the device."""
+    from rubiks_cube_solver_b200.mcts_batch import _Tree
+    buf = (ctypes.c_uint8 * 4096)()
+    base = (ctypes.addressof(buf) + 63) & ~63
+    ptrs = [name for name, _ in _Tree._fields_[4:]]
+    row_vec = ("P", "W", "N", "L")
+    word = ("node_key", "child_key", "root_key", "root_state", "leaf_state", "path_node", "path_action", "n_nodes",
+            "rand_ptr", "path_len", "flags", "sim_counter")
+    # update(size, tree, leaf_key, child_key_new, child_done_new, value, policy, value_min, sim_index, actions_out,
+    #        n_actions, n_sims, n_active, stream)
+    upd_required = (2, 3, 4, 5, 6, 9, 10, 11)
+    upd_word = (2, 3, 5, 6, 10, 11, 12)
+
+    def tree(**over):
+        t = _Tree(3, 9, 36, 36, *[base + 64 * i for i in range(len(ptrs))])
+        for name, v in over.items():
+            setattr(t, name, v)
+        return t
+
+    def traverse(size, t):
+        return lib.cube_mcts_traverse(size, ctypes.byref(t), ctypes.c_float(1.0), 150, None)
+
+    def update(size, t, over=None):
+        p = [ctypes.c_void_p(base + 2048 + 64 * i) for i in range(10)]
+        args = [size, ctypes.byref(t), p[0], p[1], p[2], p[3], p[4], ctypes.c_float(-10.0), 0, p[5], p[6], p[7], p[8], None]
+        for i, v in (over or {}).items():
+            args[i] = v
+        return lib.cube_mcts_update(*args)
+
+    for size in (2, 3):
+        for name in ptrs:
+            if name == "sim_counter":
+                continue
+            assert traverse(size, tree(**{name: None})) == _lib.CUBE_ERR_ARG, (size, name)
+            assert update(size, tree(**{name: None})) == _lib.CUBE_ERR_ARG, (size, name)
+        for i in upd_required:
+            assert update(size, tree(), {i: None}) == _lib.CUBE_ERR_ARG, (size, i)
+        offsets = {name: (1, 2) for name in word}
+        offsets.update({name: (4, 8) if size == 3 else (4,) for name in row_vec})
+        offsets["child_slot"] = (1,)
+        for name, ks in offsets.items():
+            for k in ks:
+                t = tree(**{name: getattr(tree(), name) + k})
+                assert traverse(size, t) == _lib.CUBE_ERR_ALIGN, (size, name, k)
+                assert update(size, t) == _lib.CUBE_ERR_ALIGN, (size, name, k)
+        for i in upd_word:
+            for k in (1, 2):
+                assert update(size, tree(), {i: ctypes.c_void_p(base + 2048 + 64 * 9 + k)}) == _lib.CUBE_ERR_ALIGN, (size, i, k)
+        # the counts are still checked first, and an empty batch needs no pointers at all
+        assert traverse(size, tree(n_slots=256)) == _lib.CUBE_ERR_ARG
+        assert traverse(size, tree(path_cap=0)) == _lib.CUBE_ERR_ARG
+        assert traverse(size, tree(n_trees=-1)) == _lib.CUBE_ERR_ARG
+        empty = _Tree(0, 9, 36, 36)
+        assert traverse(size, empty) == 0
+        assert lib.cube_mcts_update(size, ctypes.byref(empty), *([None] * 5), ctypes.c_float(-10.0), 0,
+                                    *([None] * 5)) == 0
+    assert lib.cube_mcts_update(3, None, *([None] * 5), ctypes.c_float(-10.0), 0, *([None] * 5)) == _lib.CUBE_ERR_ARG
+    assert b"cube_mcts_update" in lib.cube_last_error()
+
+
 def test_generated_cuda_tables_are_current():
     subprocess.check_call([sys.executable, os.path.join(ROOT, "rubiks_cube_solver_b200", "csrc", "gen_tables.py"),
                            "--check"])

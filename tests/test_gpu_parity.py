@@ -681,10 +681,13 @@ def test_batched_mcts_matches_reference_golden(size):
     assert out["solved"].any() and not out["solved"].all()
 
 
-@pytest.mark.parametrize("size", SIZES)
-def test_batched_mcts_matches_oracle_more_cases(size):
+@pytest.mark.parametrize("size,consts", [pytest.param(2, None, id="2"), pytest.param(3, None, id="3")] + [
+    pytest.param(size, consts, id="%d-cpuct%g-vl%d-vmin%g-cap%d" % ((size,) + consts))
+    for size in SIZES for consts in ((0.37, 160, -3.5, 105), (2.5, 1000, 0.25, 107))])
+def test_batched_mcts_matches_oracle_more_cases(size, consts):
     """More cubes, fewer simulations, against oracle/mcts_ref.py (itself pinned to the reference by
-    tests/test_oracle.py): ragged batch sizes and cubes solved at different simulations."""
+    tests/test_oracle.py): ragged batch sizes and cubes solved at different simulations.  `consts` =
+    (cpuct, virtual_loss_const, value_min, path_cap) other than the defaults, the path_cap not a multiple of 4."""
     import random
     from rubiks_cube_solver_b200 import mcts_batch
     from oracle import mcts_ref
@@ -697,19 +700,24 @@ def test_batched_mcts_matches_oracle_more_cases(size):
     roots = np.stack([O.scramble(size, rng.randint(A, size=(1, int(d))))[0] for d in depths])
     gpu_net = ExactSearchNet(T.STATE_DIM[size], A).to(dev())
     cpu_net = ExactSearchNet(T.STATE_DIM[size], A)
-    out = mcts_batch.BatchedMCTS(gpu_net, size, num_sim=num_sim).run(cu(roots), seeds=list(range(n)))
+    kw, search_kw = {}, {}
+    if consts is not None:
+        kw = dict(cpuct=consts[0], loss_constant=consts[1], value_min=consts[2])
+        search_kw = dict(cpuct=consts[0], virtual_loss_const=consts[1], value_min=consts[2], path_cap=consts[3])
+    out = mcts_batch.BatchedMCTS(gpu_net, size, num_sim=num_sim, **search_kw).run(cu(roots), seeds=list(range(n)))
     env = ScalarCubeEnv(size)
     for i in range(n):
         env.sim_cube = roots[i].astype(np.int64)
         env.cube = env._observe(env.sim_cube)
         with torch.no_grad():
-            acts, used, tree = mcts_ref.solve(cpu_net.predict, env, env.cube, num_sim, random.Random(i))
+            acts, used, tree = mcts_ref.solve(cpu_net.predict, env, env.cube, num_sim, random.Random(i), **kw)
         k = int(out["n_actions"][i])
         assert out["actions"][i, :k].tolist() == (acts or []), i
         assert int(out["n_sims"][i]) == used and int(out["n_nodes"][i]) == len(tree.nodes), i
         root = tree.nodes[tree.key(env.cube)]
         assert out["root_N"][i].tolist() == [int(v) for v in root[3]], i
         assert out["root_W"][i].tolist() == [float(v) for v in root[2]], i
+        assert out["root_L"][i].tolist() == [int(v) for v in root[4]], i
 
 
 def test_new_entry_points_edge_cases():
