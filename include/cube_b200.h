@@ -320,6 +320,63 @@ int cube_distance(int cube_size, const uint8_t* table, const uint8_t* states, in
 int cube_solve_optimal(int cube_size, const uint8_t* table, const uint8_t* states, int64_t n, uint8_t* actions_out,
                        uint8_t* length, void* stream);
 
+/* ---- 3x3x3 pattern databases: distance lower bounds and bounded optimal solving ----------------------------------
+ * The 3x3x3's 4.3e19 states are out of reach of a full table.  What the DeepCube line of work grades a solver with
+ * instead: admissible lower bounds from pattern databases (Korf) -- a corner table and two 6-edge tables -- and proven
+ * optimal solutions, found by IDA* guided by those bounds, for the scrambles a learned policy actually solves
+ * (test.py:103-158, train.py:167-198 measure the solve percentage only).
+ *
+ * Layout: one caller-owned uint8 buffer of cube_pattern_tables_bytes(3) = 173 335 680 bytes, three sections of one
+ * distance byte per rank.  With (p_q, o_q) = the piece and orientation of slot q in the EXACT encoding
+ * (CUBE_ENCODING_EXACT: corners q = 0..7, edges q = 0..11, the pairs cube_encode builds its columns from):
+ *   corners  offset 0            88 179 840 ranks  Lehmer(p_0..p_7) * 2187 + sum_{q<7} o_q * 3^(6-q)   (o_7 implied)
+ *   edges A  offset  88 179 840  42 577 920 ranks  pieces k = 0..5 (UB UL UF UR DB DL): mixed radix 12 * 11 * .. * 7
+ *                                                  over the slots of pieces k, each counted among the slots not yet
+ *                                                  taken, then * 64 + the six flips in base 2 (piece 0 first)
+ *   edges B  offset 130 757 760  42 577 920 ranks  the same for pieces 6..11 (DF DR FL FR BR BL), slots relabelled
+ *                                                  s -> (s - 6) mod 12
+ * The solved cube is rank 0 in every section; a section's value is the quarter-turn distance of its pattern.
+ * cube_size 2 returns CUBE_ERR_SIZE (the 2x2x2 has its exact table, cube_distance_*).  A NULL table or states
+ * pointer, n < 0, max_length outside 0..CUBE_SOLVE_BOUNDED_MAX_LENGTH or max_nodes < 0 returns CUBE_ERR_ARG.  The
+ * table and the sticker rows start on 16-byte boundaries, `nodes` on 8; the byte outputs may start anywhere. */
+#define CUBE_PATTERN_MAX_CORNERS 14      /* quarter-turn diameter of the corner pattern */
+#define CUBE_PATTERN_MAX_EDGES 11        /* ... and of either 6-edge pattern */
+#define CUBE_SOLVE_BOUNDED_MAX_LENGTH 20
+
+/* bytes of the table buffer: 173 335 680 for cube_size 3 */
+int64_t cube_pattern_tables_bytes(int cube_size);
+
+/* Fill tables [cube_pattern_tables_bytes] (caller-owned): a level-synchronous breadth-first search from the solved
+ * cube per section, four memsets and one launch per level and section. */
+int cube_pattern_tables_build(int cube_size, uint8_t* tables, void* stream);
+
+/* The admissible quarter-turn lower bound of every row (test.py:103-158, train.py:167-198: what an optimal solution
+ * can be no shorter than):
+ *   states [n, 54] uint8 in
+ *   bound  [n]     uint8 out  h = max(corners, edges A, edges B), plus 1 when h's parity differs from the corner
+ *                             permutation's (every quarter turn is a 4-cycle of corners); 255 for an unreachable row
+ *                             (a moved centre, colours that are no cubie, a piece twice, a twisted corner, a flipped
+ *                             edge, or unequal corner and edge permutation parities)
+ *   parts  [n, 3]  uint8 out or NULL: the three section values (255 for an unreachable row) */
+int cube_distance_bound(int cube_size, const uint8_t* tables, const uint8_t* states, int64_t n, uint8_t* bound,
+                        uint8_t* parts_or_null, void* stream);
+
+/* Proven optimal solutions of the rows within a budget (test.py:103-158, train.py:167-198: the optimal length
+ * beside the solve percentage): IDA* with one thread per row, thresholds from the bound in steps of 2 up to
+ * max_length, children in increasing action index over canonical quarter-turn sequences (no a ^ 1 right after a; a
+ * face twice in a row only as two equal clockwise turns, never three times; after face f no opposite face f' < f,
+ * faces U F R D B L = a >> 1).  The solution returned is the first one in that order.
+ *   actions [n, max_length] uint8  out  the solution padded with CUBE_NOOP (cube_walk of the row with it ends solved)
+ *   length  [n]             uint8  out  the optimal length, or 255 when it was not proven
+ *   lower   [n]             uint8  out  the best proven lower bound: the bound, t + 2 after each completed threshold
+ *                                       t, the length once solved; > max_length when max_length cut the search, 255
+ *                                       for an unreachable row
+ *   nodes   [n]             int64  out or NULL: child states generated (each costs a bound); a row stops, unproven,
+ *                                       before the child that would make it more than max_nodes */
+int cube_solve_bounded(int cube_size, const uint8_t* tables, const uint8_t* states, int64_t n, int max_length,
+                       int64_t max_nodes, uint8_t* actions, uint8_t* length, uint8_t* lower, int64_t* nodes_or_null,
+                       void* stream);
+
 /* ---- host-buffer front end (end-to-end path) ------------------------------------------
  * For callers that hold NumPy / host arrays, as every caller of the reference does
  * (train.py:155, :186; test.py:123).  A pipeline handle owns a few stages of device

@@ -16,6 +16,7 @@ SYMBOLS = (
     "cube_pipeline_create", "cube_pipeline_destroy", "cube_pipeline_scramble_host", "cube_pipeline_reset_host", "cube_host_alloc", "cube_host_free",
     "cube_env_host_create", "cube_env_host_destroy", "cube_env_host_step", "cube_env_host_scramble", "cube_env_host_encode",
     "cube_distance_table_entries", "cube_distance_table_build", "cube_distance", "cube_solve_optimal",
+    "cube_pattern_tables_bytes", "cube_pattern_tables_build", "cube_distance_bound", "cube_solve_bounded",
 )
 
 ABI_VERSION = 2
@@ -23,6 +24,7 @@ CUBE_ERR_SIZE, CUBE_ERR_ARG, CUBE_ERR_ALIGN, CUBE_ERR_ACTION = -1, -2, -3, -4
 DTYPE_BF16, DTYPE_F32, DTYPE_U8 = 0, 1, 2
 ENCODING_REFERENCE, ENCODING_EXACT = 0, 1
 DISTANCE_UNREACHABLE, DISTANCE_MAX_2 = 255, 14
+PATTERN_MAX_CORNERS, PATTERN_MAX_EDGES, SOLVE_BOUNDED_MAX_LENGTH = 14, 11, 20
 
 _lib = None
 
@@ -92,10 +94,15 @@ def load():
     lib.cube_distance_table_build.argtypes = [ci, vp, vp]
     lib.cube_distance.argtypes = [ci, vp, vp, i64, vp, vp]
     lib.cube_solve_optimal.argtypes = [ci, vp, vp, i64, vp, vp, vp]
+    lib.cube_pattern_tables_bytes.argtypes = [ci]
+    lib.cube_pattern_tables_build.argtypes = [ci, vp, vp]
+    lib.cube_distance_bound.argtypes = [ci, vp, vp, i64, vp, vp, vp]
+    lib.cube_solve_bounded.argtypes = [ci, vp, vp, i64, ci, i64, vp, vp, vp, vp, vp]
     for name in SYMBOLS:
         if name not in ("cube_last_error",):
             getattr(lib, name).restype = ci
     lib.cube_distance_table_entries.restype = i64
+    lib.cube_pattern_tables_bytes.restype = i64
     if lib.cube_abi_version() != ABI_VERSION:
         raise CubeLibraryError("libcube_b200.so has ABI version %d, expected %d" % (lib.cube_abi_version(), ABI_VERSION))
     _lib = lib

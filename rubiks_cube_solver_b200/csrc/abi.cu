@@ -7,6 +7,7 @@
 #include "../../include/cube_b200.h"
 #include "cube_common.cuh"
 #include "cube_distance.cuh"
+#include "cube_pattern.cuh"
 #include "cube_kernels.h"
 #include "cube_launch.cuh"
 
@@ -38,6 +39,12 @@ inline bool misaligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) 
 int fail_distance_size(const char* what)
 {
     snprintf(t_err, sizeof(t_err), "%s: exact distances exist for cube_size 2 only", what);
+    return CUBE_ERR_SIZE;
+}
+// the pattern databases exist for the 3x3x3 only
+int fail_pattern_size(const char* what)
+{
+    snprintf(t_err, sizeof(t_err), "%s: pattern databases exist for cube_size 3 only (the 2x2x2 has its exact table)", what);
     return CUBE_ERR_SIZE;
 }
 #define CUBE_DONE(fn, rc) do { int rc_ = (rc); return rc_ ? fail(rc_, fn) : 0; } while (0)
@@ -313,6 +320,43 @@ int cube_solve_optimal(int cube_size, const uint8_t* table, const uint8_t* state
     if (misaligned(table) || misaligned(states)) return fail(CUBE_ERR_ALIGN, "cube_solve_optimal");
     CUBE_DONE("cube_solve_optimal", cube::launch_solve_optimal2(table, states, n, actions_out, length,
                                                                 (cudaStream_t)stream));
+}
+
+int64_t cube_pattern_tables_bytes(int cube_size)
+{
+    if (cube_size != 3) return fail_pattern_size("cube_pattern_tables_bytes");
+    return (int64_t)kPat3Bytes;
+}
+
+int cube_pattern_tables_build(int cube_size, uint8_t* tables, void* stream)
+{
+    if (cube_size != 3) return fail_pattern_size("cube_pattern_tables_build");
+    if (!tables) return fail(CUBE_ERR_ARG, "cube_pattern_tables_build");
+    if (misaligned(tables)) return fail(CUBE_ERR_ALIGN, "cube_pattern_tables_build");
+    CUBE_DONE("cube_pattern_tables_build", cube::launch_pattern_build3(tables, (cudaStream_t)stream));
+}
+
+int cube_distance_bound(int cube_size, const uint8_t* tables, const uint8_t* states, int64_t n, uint8_t* bound,
+                        uint8_t* parts_or_null, void* stream)
+{
+    if (cube_size != 3) return fail_pattern_size("cube_distance_bound");
+    if (!tables || !states || n < 0 || (n > 0 && !bound)) return fail(CUBE_ERR_ARG, "cube_distance_bound");
+    if (misaligned(tables) || misaligned(states)) return fail(CUBE_ERR_ALIGN, "cube_distance_bound");
+    CUBE_DONE("cube_distance_bound", cube::launch_distance_bound3(tables, states, n, bound, parts_or_null,
+                                                                  (cudaStream_t)stream));
+}
+
+int cube_solve_bounded(int cube_size, const uint8_t* tables, const uint8_t* states, int64_t n, int max_length,
+                       int64_t max_nodes, uint8_t* actions, uint8_t* length, uint8_t* lower, int64_t* nodes_or_null,
+                       void* stream)
+{
+    if (cube_size != 3) return fail_pattern_size("cube_solve_bounded");
+    if (!tables || !states || n < 0 || max_length < 0 || max_length > CUBE_SOLVE_BOUNDED_MAX_LENGTH || max_nodes < 0 ||
+        (n > 0 && ((max_length > 0 && !actions) || !length || !lower)))
+        return fail(CUBE_ERR_ARG, "cube_solve_bounded");
+    if (misaligned(tables) || misaligned(states) || misaligned8(nodes_or_null)) return fail(CUBE_ERR_ALIGN, "cube_solve_bounded");
+    CUBE_DONE("cube_solve_bounded", cube::launch_solve_bounded3(tables, states, n, max_length, max_nodes, actions, length,
+                                                                lower, (long long*)nodes_or_null, (cudaStream_t)stream));
 }
 
 }  // extern "C"

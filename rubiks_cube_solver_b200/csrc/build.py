@@ -9,8 +9,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.dirname(HERE)
 LIB = os.path.join(PKG, "libcube_b200.so")
-SOURCES = ["scramble.cu", "prefix.cu", "walk.cu", "launch.cu", "expand.cu", "leaf.cu", "decode.cu", "adi.cu", "seeds.cu", "mcts.cu", "pipeline.cu", "envhost.cu", "peer.cu", "distance.cu", "abi.cu"]
-HEADERS = ["cube_common.cuh", "cube_threads.cuh", "cube_bulk.cuh", "cube_sched.cuh", "cube_launch.cuh", "cube_tables.cuh", "cube_distance.cuh", "cube_seeds.cuh", "cube_kernels.h", os.path.join("..", "..", "include", "cube_b200.h")]
+SOURCES = ["scramble.cu", "prefix.cu", "walk.cu", "launch.cu", "expand.cu", "leaf.cu", "decode.cu", "adi.cu", "seeds.cu", "mcts.cu", "pipeline.cu", "envhost.cu", "peer.cu", "distance.cu", "pattern.cu", "abi.cu"]
+HEADERS = ["cube_common.cuh", "cube_threads.cuh", "cube_bulk.cuh", "cube_sched.cuh", "cube_launch.cuh", "cube_tables.cuh", "cube_distance.cuh", "cube_pattern.cuh", "cube_seeds.cuh", "cube_kernels.h", os.path.join("..", "..", "include", "cube_b200.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-shared"]
 

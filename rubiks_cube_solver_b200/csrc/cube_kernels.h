@@ -82,6 +82,14 @@ int launch_distance2(const uint8_t* table, const uint8_t* states, long long n, u
 int launch_solve_optimal2(const uint8_t* table, const uint8_t* states, long long n, uint8_t* actions, uint8_t* length,
                           cudaStream_t stream);
 
+// 3x3x3 pattern databases (pattern.cu, layout in cube_pattern.cuh): the BFS build of the three sections (memsets and
+// one launch per level), the bound and the bounded IDA* solve
+int launch_pattern_build3(uint8_t* tables, cudaStream_t stream);
+int launch_distance_bound3(const uint8_t* tables, const uint8_t* states, long long n, uint8_t* bound, uint8_t* parts,
+                           cudaStream_t stream);
+int launch_solve_bounded3(const uint8_t* tables, const uint8_t* states, long long n, int max_length, long long max_nodes,
+                          uint8_t* actions, uint8_t* length, uint8_t* lower, long long* nodes, cudaStream_t stream);
+
 // one-shot SUM all-reduce of int64 values over peer-mapped exchange buffers (peer.cu)
 size_t peer_buffer_bytes(int cap);
 int launch_peer_allreduce_i64(int world, int rank, const uint64_t* peer_bufs, long long* values, int n, int cap,

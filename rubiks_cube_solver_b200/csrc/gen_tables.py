@@ -398,6 +398,15 @@ for _q, _d in enumerate(EDGE_DEFS_REF):
         STICKER_SLOT_3X[_s] = (8 + _q) | _k << 5
 
 
+# 3x3x3 pattern databases (csrc/cube_pattern.cuh): the cubies of the exact encoding -- corner slot q = the stickers
+# CORNER_DEFS_EXACT[q], edge slot q = EDGE_DEFS_REF[q], byte = piece | ori << 4, a piece at ori o showing
+# np.roll(home colours, o).  A turn moves the byte of slot src into slot q and adds (n - rot) mod n to its ori.
+_P_CSRC_3, _P_CROT_3 = cubie_action(MOVES_3, CORNER_DEFS_EXACT)
+_P_ESRC_3, _P_EROT_3 = cubie_action(MOVES_3, EDGE_DEFS_REF)
+PAT_MOVE_3 = [[int(_P_CSRC_3[a][q]) | ((3 - int(_P_CROT_3[a][q])) % 3) << 4 for q in range(8)]
+              + [int(_P_ESRC_3[a][q]) | ((2 - int(_P_EROT_3[a][q])) % 2) << 4 for q in range(12)] for a in range(12)]
+
+
 def hash_defs_3x():
     words = [_bytes([d[0], d[1], d[2], 0]) for d in CORNER_DEFS_EXACT]
     words += [_bytes([d[0], d[1], d[1], 1]) for d in EDGE_DEFS_REF]
@@ -624,6 +633,9 @@ def render():
              "// [3 * cubelet + ori] = the colours of the slot's stickers k = 0..2, one per byte\n")
     o.append(_c_array("uint8_t", "kDistMove2", DIST_MOVE_2, per_line=21, fmt="%d"))
     o.append(_c_array("uint32_t", "kCubieColours2", CUBIE_COLOURS_2, per_line=7))
+    o.append("// 3x3x3 pattern databases (cube_pattern.cuh): [move][slot] = source slot | ori added << 4, corner slots\n"
+             "// 0..7 then edge slots 0..11, in the cubies of the exact encoding\n")
+    o.append(_c_array("uint8_t", "kPatMove3", [v for r in PAT_MOVE_3 for v in r], per_line=20, fmt="%d"))
     return "".join(o)
 
 
@@ -755,6 +767,22 @@ def selftest(n=300, depth=37):
             "2x2x2 distance cubies disagree with getOP"
         assert all(CUBIE_COLOURS_2[3 * (c & 15) + (c >> 4)] == sum(int(s[d[k]]) << (8 * k) for k in range(3))
                    for c, d in zip(codes, PIECE_DEFS_2)), "kCubieColours2 does not rebuild the stickers"
+    # pattern-database cubies: a turn through kPatMove3 equals the exact encoding of the turned stickers
+    def exact_cubies(s):
+        c = [CORNER_COL_3X[s[d[0]] + 2 * s[d[1]] + 10 * s[d[2]]] for d in CORNER_DEFS_EXACT]
+        e = [EDGE_COL_3[s[d[0]] + 10 * s[d[1]]] for d in EDGE_DEFS_REF]
+        return [v // 3 | (v % 3) << 4 for v in c] + [v // 2 | (v % 2) << 4 for v in e]
+    for _ in range(n):
+        s = np.repeat(np.arange(6), 9)
+        cub = exact_cubies(s)
+        assert cub == list(range(8)) + list(range(12)), "the solved cube must be piece q in slot q, ori 0"
+        for m in rng.randint(12, size=depth):
+            s = s[MOVES_3[m]]
+            row = PAT_MOVE_3[m]
+            cub = [(cub[row[q] & 15] & 15) | (((cub[row[q] & 15] >> 4) + (row[q] >> 4)) % 3) << 4 for q in range(8)] + \
+                  [(cub[8 + (row[q] & 15)] & 15) | (((cub[8 + (row[q] & 15)] >> 4) + (row[q] >> 4)) % 2) << 4
+                   for q in range(8, 20)]
+        assert cub == exact_cubies(s), "3x3x3 pattern cubies disagree with the exact encoding"
     # cycles reproduce the gather rows
     for moves, cycles, n_s in ((MOVES_3, CYCLES_3, 54), (MOVES_2, CYCLES_2, 24)):
         for m in range(len(moves)):

@@ -460,6 +460,93 @@ def solve_optimal(cube_size, states):
     return actions, length
 
 
+_pattern_tables = {}
+_pattern_lock = threading.Lock()
+
+# Per-row node budget of solve_bounded.  On seeded scrambles of depth 8 / 10 / 12 / 14 (4 096 each) the search needed
+# at most 893 / 3 943 / 63 570 / 2 157 028 child states (tools/distance_333.py, profiles/r04_distance_333.json; B200,
+# 1 000 W), so 4 Mi proves all of them with room to spare.  A row runs in one thread, which generated at least 0.45 M
+# children per second there (2.16 M within the 4.76 s call): one row that exhausts 4 Mi holds a call about 9 s.
+SOLVE_BOUNDED_MAX_NODES = 1 << 22
+
+
+def _pattern_bytes(cube_size):
+    _geom(cube_size)
+    n = _lib.load().cube_pattern_tables_bytes(cube_size)
+    if n < 0:
+        _lib.check(n, "cube_pattern_tables_bytes")                        # 2x2x2: NotImplementedError
+    return n
+
+
+def pattern_tables(device=None):
+    """The 3x3x3 pattern databases (C ABI cube_pattern_tables_build): uint8 [173335680], the corner table and the two
+    6-edge tables (layout in include/cube_b200.h).  Built on the device the first time they are asked for there,
+    then cached per device; treat them as read-only."""
+    dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    if dev.type != "cuda":
+        raise TypeError("pattern_tables live on a CUDA device (this library has no CPU path)")
+    if dev.index is None:
+        dev = torch.device("cuda", torch.cuda.current_device())
+    with _pattern_lock:
+        tables = _pattern_tables.get(dev.index)
+        if tables is None:
+            lib = _lib.load()
+            tables = torch.empty(_pattern_bytes(3), dtype=torch.uint8, device=dev)
+            with torch.cuda.device(dev):
+                _lib.check(lib.cube_pattern_tables_build(3, _ptr(tables), _stream(dev)), "cube_pattern_tables_build")
+                torch.cuda.current_stream(dev).synchronize()              # once: callers on any stream may read them
+            _pattern_tables[dev.index] = tables
+    return tables
+
+
+def _pattern_rows(cube_size, states):
+    _pattern_bytes(cube_size)
+    states = _require_cuda(states, "states")
+    n = states.shape[0]
+    if states.shape != (n, N_STICKERS[cube_size]):
+        raise ValueError("states must be [N, %d]" % N_STICKERS[cube_size])
+    return states, n, pattern_tables(states.device)
+
+
+def distance_bound(cube_size, states, parts=False):
+    """Admissible quarter-turn lower bound of every sticker row (C ABI cube_distance_bound): uint8 [N], 255 for a
+    row that is not a reachable state; with parts=True also the corner, edges-A and edges-B values, uint8 [N, 3].
+    3x3x3 only (2x2x2 raises NotImplementedError: use `distance`)."""
+    states, n, tables = _pattern_rows(cube_size, states)
+    dev = states.device
+    bound = torch.empty(n, dtype=torch.uint8, device=dev)
+    p = torch.empty((n, 3), dtype=torch.uint8, device=dev) if parts else None
+    if n:
+        with torch.cuda.device(dev):
+            _lib.check(_lib.load().cube_distance_bound(cube_size, _ptr(tables), _ptr(states), n, _ptr(bound), _ptr(p),
+                                                       _stream(dev)), "cube_distance_bound")
+    return (bound, p) if parts else bound
+
+
+def solve_bounded(cube_size, states, max_length=14, max_nodes=SOLVE_BOUNDED_MAX_NODES, want_nodes=False):
+    """Proven optimal solutions within a budget (C ABI cube_solve_bounded): IDA* over the pattern-database bound, one
+    thread per row.  Returns (actions uint8 [N, max_length] padded with the no-op index 12, length uint8 [N] = the
+    optimal length or 255 where it was not proven, lower uint8 [N] = the best proven lower bound[, nodes int64 [N]]).
+    A row is unproven when the search reached max_length (lower > max_length) or generated max_nodes children;
+    `walk(cube_size, states, actions)` ends solved for every proven row.  3x3x3 only."""
+    if not 0 <= max_length <= _lib.SOLVE_BOUNDED_MAX_LENGTH:
+        raise ValueError("max_length must be in 0..%d" % _lib.SOLVE_BOUNDED_MAX_LENGTH)
+    if max_nodes < 0:
+        raise ValueError("max_nodes must be >= 0")
+    states, n, tables = _pattern_rows(cube_size, states)
+    dev = states.device
+    actions = torch.empty((n, max_length), dtype=torch.uint8, device=dev)
+    length = torch.empty(n, dtype=torch.uint8, device=dev)
+    lower = torch.empty(n, dtype=torch.uint8, device=dev)
+    nodes = torch.empty(n, dtype=torch.int64, device=dev) if want_nodes else None
+    if n:
+        with torch.cuda.device(dev):
+            _lib.check(_lib.load().cube_solve_bounded(cube_size, _ptr(tables), _ptr(states), n, max_length, max_nodes,
+                                                      _ptr(actions), _ptr(length), _ptr(lower), _ptr(nodes),
+                                                      _stream(dev)), "cube_solve_bounded")
+    return (actions, length, lower, nodes) if want_nodes else (actions, length, lower)
+
+
 class HostCube(object):
     """One cube per call through host (NumPy) buffers -- C ABI cube_env_host_*: the per-call path of the
     drop-in CubeEnv (reset / step / get_obs, cube_env.py:56-147).  Two launches and one stream

@@ -119,29 +119,44 @@ def validation(model, cube_size, sample_scramble_count=30, sample_cube_count=10,
     return [float(x) for x in solved.cpu()]
 
 
-def optimal_gap(model, seeds, depths, max_timesteps=200, mask_inverse=False, model_device=None):
-    """How far the greedy policy's 2x2x2 solutions are from optimal: `validation`'s solve-% curve with the
-    solution-length comparison beside it.  Every (depth, seed) cube is scrambled as reset(seed, depth) draws it and
-    solved by `greedy_solve`; the exact distance of every scramble comes from the distance table (ops.distance).
+def optimal_gap(model, seeds, depths, max_timesteps=200, mask_inverse=False, model_device=None, cube_size=2):
+    """How far the greedy policy's solutions are from optimal: `validation`'s solve-% curve with the solution-length
+    comparison beside it.  Every (depth, seed) cube is scrambled as reset(seed, depth) draws it and solved by
+    `greedy_solve`.  2x2x2: the exact distance of every scramble comes from the distance table (ops.distance).
+    3x3x3: from ops.solve_bounded, which proves the distance of a scramble within its default length and node budget
+    and gives a lower bound for the rest.
 
-    Returns one dict per depth: depth, solved_pct, mean_distance (over all cubes), mean_steps (over the cubes
-    greedy solved) and mean_excess (steps - distance over the cubes greedy solved, leaving out scrambles that
-    already end solved: greedy counts those only after stepping back, see the module docstring).  A mean over no
-    cube is NaN."""
+    Returns one dict per depth: depth, solved_pct, mean_distance, mean_steps (over the cubes greedy solved) and
+    mean_excess (steps - distance over the cubes greedy solved, leaving out scrambles that already end solved: greedy
+    counts those only after stepping back, see the module docstring).  For the 2x2x2, mean_distance is over all
+    cubes.  For the 3x3x3, mean_distance and mean_excess are over the cubes whose distance was proven, and each dict
+    adds proven_pct and mean_lower_bound (over all cubes).  A mean over no cube is NaN."""
     seeds, depths = [int(s) for s in seeds], [int(d) for d in depths]
-    moves = reference_scrambles_device(2, seeds, depths)
-    res = greedy_solve(model, 2, moves, max_timesteps=max_timesteps, mask_inverse=mask_inverse,
+    moves = reference_scrambles_device(cube_size, seeds, depths)
+    res = greedy_solve(model, cube_size, moves, max_timesteps=max_timesteps, mask_inverse=mask_inverse,
                        model_device=model_device)
-    start, _, _ = ops.scramble(2, moves, want_flags=False)
+    start, _, _ = ops.scramble(cube_size, moves, want_flags=False)
     shape = (len(depths), len(seeds))
-    dist = ops.distance(2, start).cpu().numpy().reshape(shape).astype(np.int64)
+    if cube_size == 3:
+        _, length, lower = ops.solve_bounded(3, start)
+        dist = length.cpu().numpy().reshape(shape).astype(np.int64)
+        lower = lower.cpu().numpy().reshape(shape).astype(np.int64)
+        proven = dist != 255
+    else:
+        dist = ops.distance(cube_size, start).cpu().numpy().reshape(shape).astype(np.int64)
+        proven = np.ones(shape, dtype=bool)
     solved = res["solved"].cpu().numpy().reshape(shape)
     steps = res["steps"].cpu().numpy().reshape(shape)
 
     def mean(x):
         return float(x.mean()) if x.size else float("nan")
 
-    return [dict(depth=d, solved_pct=float(solved[i].mean()) * 100.0, mean_distance=mean(dist[i]),
-                 mean_steps=mean(steps[i][solved[i]]),
-                 mean_excess=mean((steps[i] - dist[i])[solved[i] & (dist[i] > 0)]))
-            for i, d in enumerate(depths)]
+    out = []
+    for i, d in enumerate(depths):
+        row = dict(depth=d, solved_pct=float(solved[i].mean()) * 100.0, mean_distance=mean(dist[i][proven[i]]),
+                   mean_steps=mean(steps[i][solved[i]]),
+                   mean_excess=mean((steps[i] - dist[i])[solved[i] & proven[i] & (dist[i] > 0)]))
+        if cube_size == 3:
+            row.update(proven_pct=float(proven[i].mean()) * 100.0, mean_lower_bound=mean(lower[i]))
+        out.append(row)
+    return out
